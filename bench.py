@@ -8,12 +8,16 @@ BASELINE.json configs[2], the configuration north_star's targets are quoted on:
     composition polynomial LDE + commitment, OOD frames, DEEP composition, FRI commit phase, PoW grinding, query
     openings and proof serialisation.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--config cfg3|cfg2]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--config cfg3|cfg2] [--dump-outputs DIR]
 
 Prints ONE JSON line (rank 0). `value` = ms per proof with the trace already resident in HBM; `e2e` = ms per proof
 through the C ABI with HOST buffers (pinned trace columns copied H2D inside the timed region, proof bytes returned
 to the host). N = 1: one GPU. N > 1: ONE proof sharded over the N GPUs (strong scaling; winterfell_b200/dist.py),
 byte-identical to the single-GPU proof. A short cfg2 (2^20 x 8, base field) record rides along as `cfg2`.
+
+`--dump-outputs DIR` writes the proofs the last timed step of each arm returned, `proof.npy` (resident) and
+`proof_e2e.npy` (e2e), one float32 per proof byte. The trace is a fixed function of the configuration, so two builds run
+with the same arguments can be compared output for output.
 
 `--impl reference` times the CPU arm: the oracle (C++ restatement of the reference's `concurrent` prover — the
 reference is Rust and cannot be built in this image) at the FULL configuration, for as many steps as fit the wall
@@ -31,6 +35,7 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True   # the benchmark writes nothing into the tree it runs from (which may be read-only)
 
 P = 0xFFFFFFFF00000001
 METRIC = "prover_ms"
@@ -312,7 +317,13 @@ def main():
     ap.add_argument("--config", default="cfg3", choices=sorted(CONFIGS))
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-sub-record", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the proofs the last timed step returned as DIR/<name>.npy (float32, one value per byte)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs:
+        os.makedirs(args.dump_outputs, exist_ok=True)   # fail on an unusable DIR before the timed run, not after it
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -347,16 +358,17 @@ def main():
         return torch.cuda.Event(enable_timing=True)
 
     def timed(fn, steps):
-        total = 0.0
+        """Mean ms per step over `steps` calls of fn, and what the last call returned."""
+        total, out = 0.0, None
         for _ in range(steps):
             flush.zero_()
             a, b = ev(), ev()
             a.record(stream)
-            fn()
+            out = fn()
             b.record(stream)
             b.synchronize()
             total += a.elapsed_time(b)
-        return total / steps
+        return total / steps, out
 
     def run_config(cfg, steps, warm, sample_clocks):
         """Resident and e2e arms of one configuration on this rank's GPU. Returns a dict."""
@@ -388,11 +400,11 @@ def main():
             barrier()
             l0 = ctx.launches
             t_wall0 = time.perf_counter()
-            ms_step = timed(step_resident, steps)
+            ms_step, last_res = timed(step_resident, steps)
             barrier()
             wall_ms = (time.perf_counter() - t_wall0) * 1e3
             launches = int(ctx.launches - l0) // max(steps, 1)
-            e2e_step = timed(step_e2e, steps)
+            e2e_step, last_e2e = timed(step_e2e, steps)
             barrier()
             if sampler:
                 sampler.stop_flag = True
@@ -405,7 +417,8 @@ def main():
             ctx.set_profiling(False)
         del dev
         return {"ms": ms_step, "e2e_ms": e2e_step, "launches": launches, "breakdown": breakdown, "proof": p_e2e, "h2d": int(host_np.nbytes),
-                "wall_ms": wall_ms / steps, "clocks": sampler.summary() if sampler else None}
+                "wall_ms": wall_ms / steps, "clocks": sampler.summary() if sampler else None,
+                "last_outputs": {"proof": last_res, "proof_e2e": last_e2e}}
 
     def fri_compressions(L):
         """BLAKE3 compressions of the FRI commit phase on an L-point base-field codeword (folding 4): every layer of n points
@@ -463,7 +476,7 @@ def main():
             main_rec["parallelism"] = f"{world} independent replicas of the proof, one per GPU (no data-path collective)"
     sub = None
     if world == 1 and args.config == "cfg3" and not args.no_sub_record:
-        sub = run_config("cfg2", max(args.steps, 10), 3, False)
+        sub = run_config("cfg2", args.steps, 3, False)
     sweep = None if args.no_sub_record else fri_sweep()
     gc.enable()
 
@@ -474,6 +487,11 @@ def main():
         ms_step, e2e_step = float(t[0]), float(t[1])
 
     if rank == 0:
+        if args.dump_outputs:
+            # the serialized proof is what a caller of the timed path receives; its bytes are exact in float32. The proof buffer
+            # holds at most 8 MiB, so the two files stay within 64 MiB.
+            for name, proof in main_rec["last_outputs"].items():
+                np.save(os.path.join(args.dump_outputs, name + ".npy"), np.frombuffer(proof, dtype=np.uint8).astype(np.float32))
         peaks = {}
         try:
             peaks = json.load(open(os.path.join(ROOT, "MEASURED_PEAKS.json")))
@@ -539,7 +557,7 @@ def main():
                 s_log_n = max(log_n - 4, 10)
                 code = ("import json,sys; sys.path.insert(0, %r); import bench; ms, steps, warm, cores = bench.cpu_prove(%d, %d, %d, 1, 0, 120.0); "
                         "print(json.dumps({'ms': ms, 'cores': cores}))" % (ROOT, pairs, s_log_n, ext))
-                out = subprocess.run([sys.executable, "-c", code], capture_output=True, text=True, timeout=600,
+                out = subprocess.run([sys.executable, "-B", "-c", code], capture_output=True, text=True, timeout=600,
                                      env={**os.environ, "OMP_WAIT_POLICY": "PASSIVE"}).stdout.strip().splitlines()[-1]
                 r = json.loads(out)
                 line["cpu_baseline"] = {"value": round(r["ms"], 3), "unit": "ms", "cores": r["cores"], "kind": "port", "rows_log2": s_log_n,

@@ -322,7 +322,7 @@ def bench_sharded(ctx, stream, cfg, steps, warmup, configs, proof_opts, flush, c
         dist.barrier()
         torch.cuda.synchronize()
 
-    step_log = {}
+    step_log, last_outputs = {}, {}
 
     def timed(fn, k, name):
         total, per = 0.0, []
@@ -331,12 +331,13 @@ def bench_sharded(ctx, stream, cfg, steps, warmup, configs, proof_opts, flush, c
             barrier()                                                    # ranks start a proof together
             a, b = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
             a.record(stream)
-            fn()
+            out = fn()
             b.record(stream)
             b.synchronize()
             per.append(a.elapsed_time(b))
             total += per[-1]
         step_log[name] = per
+        last_outputs[name] = out
         return total / k
 
     with torch.cuda.stream(stream):
@@ -382,6 +383,7 @@ def bench_sharded(ctx, stream, cfg, steps, warmup, configs, proof_opts, flush, c
     bd_ex = breakdown.get("trace_exchange", 0.0)
     return {"ms": ms, "e2e_ms": e2e, "launches": launches, "breakdown": breakdown, "proof": proof, "h2d": int(host_np.nbytes) * world,
             "wall_ms": wall, "clocks": sampler.summary(),
+            "last_outputs": {"proof": last_outputs["resident"], "proof_e2e": last_outputs["e2e"]},
             "parallelism": f"one proof sharded over {world} GPUs: column-sharded interpolate + LDE, exchange into row shards, row-sharded "
                            "commitments / constraints / DEEP / first FRI layers, subtree-root all-gathers (winterfell_b200/dist.py)",
             "comm": {"limiting_collective": ("column shards -> row shards of the trace LDE fused into the LDE: the last pass of every coset's transform stores each "
