@@ -272,7 +272,7 @@ int wf_grind(wf_ctx* ctx, int hash_id, const uint8_t seed[32], uint32_t grinding
 /* ---- one proof sharded over several GPUs (SURVEY.md 8e; one process and one wf_ctx per GPU) ------------------
  * The reference has no distributed prover; its unit of distribution is the column (ColMatrix columns are independent,
  * prover/src/matrix/col_matrix.rs:192-202) and PartitionOptions (air/src/options.rs:405-445). Here rank r of `world`
- * owns trace columns [r*w/world, (r+1)*w/world): it interpolates and extends them locally, the LDE is exchanged into
+ * owns a block of whole 8-column segments of the trace (wf_host_shard_columns): it interpolates and extends them locally, the LDE is exchanged into
  * row shards (rank r holds LDE rows [r*N/world, (r+1)*N/world) of ALL columns plus `blowup` halo rows), and leaf
  * hashing, constraint evaluation, DEEP composition and the first FRI layers run on row shards; every Merkle tree is a
  * local subtree per rank plus log2(world) top levels built from an all-gather of the subtree roots; query openings are
@@ -311,6 +311,24 @@ typedef struct wf_comm {
 int wf_prove_fib_sharded(wf_ctx* ctx, const wf_comm* comm, const uint64_t* const* local_cols, const uint64_t* d_local, int mont,
                          uint32_t k, uint32_t log_n, const uint64_t* results, const uint32_t* opts, uint8_t* proof,
                          size_t* proof_len, double* stats);
+/* Which trace columns rank `rank` of `world` owns in a sharded proof: the S = ceil(width / 8) segments are split
+ * as evenly as possible. Rank r owns segments [floor(r S / world), floor((r+1) S / world)), which gives columns
+ * [*first, *first + *count); *count may be 0. When 8 * world divides the width, these are the blocks wf_prove_fib_sharded
+ * takes. width 1..255, world a power of two >= 2, 0 <= rank < world; WF_OK or WF_ERR_INVALID. Host-only. */
+int wf_host_shard_columns(uint32_t width, int world, int rank, uint32_t* first, uint32_t* count);
+/* wf_prove_air (single-segment description) sharded over comm->world GPUs. This rank passes the columns
+ * wf_host_shard_columns names: host columns, or d_local = device column-major [count][2^log_n]; a rank that owns no
+ * column passes NULL for both (it still takes part in every collective). air_desc, log_n and opts are the whole proof's
+ * and must be the same on every rank. Every rank returns the same bytes, equal to wf_prove_air's on one GPU.
+ * Before any device work every rank checks its own arguments (description, no aux segment: WF_ERR_UNSUPPORTED; world a
+ * power of two >= 2; columns passed iff some are owned; blowup >= the constraints' blowup; at least 64 * blowup LDE rows and
+ * 64 constraint-evaluation rows per rank) and the ranks all-gather (status, hash of description, log_n, opts, world): if
+ * any rank refused, every rank returns the lowest refusing rank's status; if the hashes differ, every rank returns
+ * WF_ERR_INVALID. No rank then waits on another. stats: as wf_prove_fib_sharded; [6] = 2 only when every rank owns the
+ * same number of whole 8-column segments (the fused form needs it; other splits take the peer copies). */
+int wf_prove_air_sharded(wf_ctx* ctx, const wf_comm* comm, const uint64_t* air_desc, size_t air_desc_len,
+                         const uint64_t* const* local_cols, const uint64_t* d_local, int mont, uint32_t log_n,
+                         const uint32_t* opts, uint8_t* proof, size_t* proof_len, double* stats);
 
 /* ---- constraint kernels compiled per AIR ---------------------------------------------------------------------------
  * wf_eval_constraints / wf_prove_air[_aux] evaluate the AIR's transition programs with a kernel compiled at run time for that

@@ -110,6 +110,9 @@ _SIGS = [
     ("wf_host_sharded_opening_plan", C.c_long, [C.c_size_t, C.c_int, C.c_int, u64p, C.c_size_t, u64p, u64p, C.c_size_t]),
     ("wf_prove_fib_sharded", C.c_int, [vp, vp, C.POINTER(u64p), vp, C.c_int, C.c_uint32, C.c_uint32, u64p, C.POINTER(C.c_uint32), u8p,
                                        C.POINTER(C.c_size_t), C.POINTER(C.c_double)]),
+    ("wf_host_shard_columns", C.c_int, [C.c_uint32, C.c_int, C.c_int, C.POINTER(C.c_uint32), C.POINTER(C.c_uint32)]),
+    ("wf_prove_air_sharded", C.c_int, [vp, vp, u64p, C.c_size_t, C.POINTER(u64p), vp, C.c_int, C.c_uint32, C.POINTER(C.c_uint32), u8p,
+                                       C.POINTER(C.c_size_t), C.POINTER(C.c_double)]),
 ]
 
 
@@ -578,6 +581,14 @@ def sharded_opening_plan(n_global, world, rank, positions):
     if cnt < 0:
         raise WfError("wf_host_sharded_opening_plan: bad arguments")
     return want[:cnt].copy(), idx[:cnt].copy()
+
+
+def shard_columns(width, world, rank):
+    """(first, count): the trace columns rank `rank` of `world` owns in a sharded proof (wf_host_shard_columns)."""
+    first, count = C.c_uint32(0), C.c_uint32(0)
+    if lib().wf_host_shard_columns(width, world, rank, C.byref(first), C.byref(count)) != WF_OK:
+        raise WfError(f"wf_host_shard_columns: bad arguments (width {width}, world {world}, rank {rank})")
+    return first.value, count.value
 
 
 def host_hash_elements(hash_id, elems):

@@ -686,7 +686,8 @@ int wf_trace_lde_from_host(wf_ctx* ctx, const uint64_t* const* cols, uint32_t nc
     return wf_trace_lde_cosetwise(ctx, cols, nullptr, ncols, nrows, mont, log_blowup, polys_out, lde_out, false, nullptr, nullptr);
 }
 // The same pipeline with two knobs for the sharded prover (prover.cu): coset_major = the LDE is written coset-major
-// (row k * n + j = P(7 w_N^k w_n^j); *lde_out must then be preallocated with the natural segment width) and after_coset(k)
+// (row k * n + j = P(7 w_N^k w_n^j); *lde_out must then be preallocated, with the natural segment width of `ncols` columns or
+// a wider one: a rank of a sharded proof writes its columns at the segment width of the whole trace) and after_coset(k)
 // is called once coset k of ALL columns has been enqueued on the ctx stream — the caller starts that coset's exchange there.
 // d_cols != NULL: the columns are already on the device (column-major), no upload stage.
 int wf_trace_lde_cosetwise(wf_ctx* ctx, const uint64_t* const* cols, const uint64_t* d_cols, uint32_t ncols, size_t nrows, int mont,
@@ -696,11 +697,13 @@ int wf_trace_lde_cosetwise(wf_ctx* ctx, const uint64_t* const* cols, const uint6
     u32 log_n;
     if (log2_exact(nrows, &log_n) || log_n < 1) return wf_fail(ctx, WF_ERR_INVALID, "rows must be a power of two >= 2");
     if (log_blowup > 7 || log_n + log_blowup > 32) return wf_fail(ctx, WF_ERR_INVALID, "bad blowup");
-    const int Wout = seg_width_for(ncols);
+    const int Wn = seg_width_for(ncols);
+    const bool prealloc = coset_major && !scatter;
+    if (prealloc && (!lde_out || !*lde_out || (*lde_out)->m.rows != (nrows << log_blowup) || (*lde_out)->m.W < Wn || (*lde_out)->m.cols != ncols))
+        return wf_fail(ctx, WF_ERR_INVALID, "coset-major output must be preallocated");
+    const int Wout = prealloc ? (*lde_out)->m.W : Wn;
     const u32 nseg_out = (ncols + Wout - 1) / Wout;
     const u32 nb = 1u << log_blowup;
-    if (coset_major && !scatter && (!*lde_out || (*lde_out)->m.rows != (nrows << log_blowup) || (*lde_out)->m.W != Wout || (*lde_out)->m.cols != ncols))
-        return wf_fail(ctx, WF_ERR_INVALID, "coset-major output must be preallocated");
     // cosets of one column chunk: all at once, or one by one with the callback when this is the last chunk
     auto extend = [&](const SegMatrix& pv, SegMatrix& ov, u32 out_col0, bool last, u32 out_seg) -> int {
         if (scatter) {  // every coset straight into the owners' row shards (natural order there); `ov` is not written
@@ -721,7 +724,7 @@ int wf_trace_lde_cosetwise(wf_ctx* ctx, const uint64_t* const* cols, const uint6
         }
         return WF_OK;
     };
-    int Wc = nseg_out >= 2 ? Wout : (Wout >= 4 ? Wout / 2 : 0);
+    int Wc = nseg_out >= 2 ? Wout : (Wn >= 4 ? Wn / 2 : 0);
     // (measured on cfg2, 8 columns: halves 7.03 ms e2e, quarters 7.35 — W = 2 tiles cost more than the
     // shorter upload head saves — no pipeline 7.36)
     if (d_cols || Wc == 0 || log_n < 12) {  // resident columns, or too narrow / too small to be worth a pipeline

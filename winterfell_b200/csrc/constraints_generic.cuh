@@ -69,6 +69,10 @@ struct GenEvalParams {
     const u64* const* ae_tab;
     const u32* ae_tstride;
     const u32* ae_shift;
+    // row-sharded evaluation (multi-GPU): this launch covers CE rows [row0, row0 + ce_rows); `lde` (and `alde`) then hold the
+    // LDE rows of that range followed by `blowup` halo rows, so the next-state row is local row + blowup without wrap-around,
+    // and `out` holds the launch's rows only. ce_rows = 0: the whole domain.
+    size_t row0, ce_rows;
 };
 
 #ifdef WF_JIT
@@ -81,11 +85,12 @@ template <int D> __device__ __forceinline__ void wf_jit_aux(GlExt<D>* ra, const 
 template <int D, bool AUX>
 __device__ __forceinline__ void generic_constraints_row(const GenEvalParams& p) {
     const size_t ce = (size_t)1 << (p.log_n + p.log_ce_blowup);
-    const size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= ce) return;
+    const size_t il = (size_t)blockIdx.x * blockDim.x + threadIdx.x;   // row of this launch: indexes lde / alde / out
+    if (il >= (p.ce_rows ? p.ce_rows : ce)) return;
+    const size_t i = il + p.row0;                                       // row of the CE domain: x, divisors, periodic and sequence tables
     const size_t N = (size_t)1 << (p.log_n + p.log_blowup);
-    const size_t ls = i << (p.log_blowup - p.log_ce_blowup);
-    const size_t nx = (ls + ((size_t)1 << p.log_blowup)) & (N - 1);
+    const size_t ls = il << (p.log_blowup - p.log_ce_blowup);
+    const size_t nx = p.ce_rows ? ls + ((size_t)1 << p.log_blowup) : ((ls + ((size_t)1 << p.log_blowup)) & (N - 1));
     GlExt<D> T = ext_zero<D>();
 #ifdef WF_JIT
     // compile-time shape: every index below is a literal after unrolling, r[] and ra[] are promoted to registers; the rows a
@@ -235,7 +240,7 @@ __device__ __forceinline__ void generic_constraints_row(const GenEvalParams& p) 
             }
         }
     }
-    u64* o = p.out.base + i * p.out.W;
+    u64* o = p.out.base + il * p.out.W;
 #pragma unroll
     for (int q = 0; q < D; q++) o[q] = acc.v[q];
 }

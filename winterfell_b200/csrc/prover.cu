@@ -731,6 +731,32 @@ struct Channel {  // ProverChannel (prover/src/channel.rs)
     }
 };
 
+// Channel seed: Context::to_elements || public inputs (prover/src/channel.rs:57-82, air/src/air/context.rs:119-136), with
+// TraceInfo::to_elements (air/src/air/trace_info.rs:209-238)
+static std::vector<u64> channel_seed(const AirHost& air, size_t n, const Options& o) {
+    const u32 c = air.w, aw = air.aw;
+    const size_t n_cons = air.degrees.size() + air.aux_degrees.size() + air.asserts.size() + air.aux_asserts.size();
+    const u64 ti0 = aw ? ((((((u64)c << 8) | 1) << 8) | aw) << 8) | air.nr : ((u64)c << 8);
+    std::vector<u64> seed = {ti0, (u64)n, 1, 0xFFFFFFFFULL, (u64)n_cons,
+                             ((u64)o.ext << 24) | ((u64)o.folding << 16) | ((u64)o.rem_max_deg << 8) | o.blowup,
+                             o.grinding, o.num_queries};
+    for (u64 v : air.pub_inputs) seed.push_back(v);
+    return seed;
+}
+// Head of the proof object (prover/src/lib.rs:464-489; air/src/proof/mod.rs:189-200): the Context (context.rs:142-151:
+// TraceInfo, modulus, ProofOptions, number of constraints), the number of query positions and the commitments
+static void write_proof_head(ByteVec& w, const AirHost& air, u32 log_n, const Options& o, size_t num_positions, const ByteVec& commitments) {
+    const size_t n_cons = air.degrees.size() + air.aux_degrees.size() + air.asserts.size() + air.aux_asserts.size();
+    w.u8_((u8)air.w); w.u8_((u8)air.aw); w.u8_((u8)air.nr); w.u8_((u8)log_n); w.u16_(0);
+    w.u8_(8); w.u64_(GL_P);
+    w.u8_((u8)o.num_queries); w.u8_((u8)o.blowup); w.u8_((u8)o.grinding); w.u8_((u8)o.ext); w.u8_((u8)o.folding);
+    w.u8_((u8)o.rem_max_deg); w.u8_((u8)o.batch_c); w.u8_((u8)o.batch_d); w.u8_((u8)o.num_partitions); w.u8_((u8)o.hash_rate);
+    w.usize(n_cons);
+    w.u8_((u8)num_positions);
+    w.u16_((uint16_t)commitments.v.size());
+    w.bytes(commitments.v.data(), commitments.v.size());
+}
+
 template <int D>
 int upload_ext(wf_ctx* ctx, const std::vector<GlExt<D>>& v, size_t first, size_t count, u64** out) {
     void* p;
@@ -875,13 +901,12 @@ template <int D>
 int eval_constraints(wf_ctx* ctx, const AirHost& air, const wf_mat* lde, const wf_mat* alde, const std::vector<GlExt<D>>& cc,
                      const std::vector<u64>& rnd_flat, u32 log_n, u32 log_b, wf_mat** out, size_t row0 = 0, size_t ce_rows = 0) {
     // ce_rows != 0: row-sharded call — CE rows [row0, row0 + ce_rows) only; `lde` then holds the LDE rows of that range
-    // followed by `blowup` halo rows (FibEvalParams::row0)
+    // followed by `blowup` halo rows (FibEvalParams::row0, GenEvalParams::row0)
     const size_t n = (size_t)1 << log_n;
     const u32 c = air.w, aw = air.aw, log_ceb = air.log_ce_blowup();
     const u32 n_atr = (u32)air.aux_degrees.size(), n_mtr = (u32)air.degrees.size(), n_mas = (u32)air.asserts.size();
     const u32 n_tr = n_mtr + n_atr;
     const size_t ce = n << log_ceb;
-    if (ce_rows && !air.is_fib) return wf_fail(ctx, WF_ERR_UNSUPPORTED, "row-sharded constraint evaluation covers the FibSmall family");
     wf_mat* comp;
     CKI(wf_mat_alloc(ctx, ce_rows ? ce_rows : ce, D, &comp));
     if (comp->m.W > D) CK(cudaMemsetAsync(comp->m.base, 0, comp->m.words() * 8, ctx->st));
@@ -1012,6 +1037,7 @@ int eval_constraints(wf_ctx* ctx, const AirHost& air, const wf_mat* lde, const w
         CKI(upload(zt.data(), zt.size() * 8, &dp)); p.zt = (const u64*)dp;
         p.num_exempt = air.exemptions;
         for (u32 e = 0; e < air.exemptions; e++) p.exempt[e] = gl_pow(g_tr, n - air.exemptions + e);  // divisor.rs:31-41
+        p.row0 = row0; p.ce_rows = ce_rows;   // run-time parameters: the compiled kernel of an AIR serves every rank
         std::vector<u32> agoff = {0}, aecol, aetstride, aeshift;
         std::vector<u64> aga, agb, agoa, aeval, aecc, fa;
         std::vector<const u64*> aetab;
@@ -1059,13 +1085,14 @@ int eval_constraints(wf_ctx* ctx, const AirHost& air, const wf_mat* lde, const w
         const bool jit = ctx->jit_enabled &&
                          wf_jit_get_kernel(ctx, wf_jit_source(D, air.w, (u32)air.periodic.size(), air.num_regs, air.prog, air.consts, aw, air.nr,
                                                               air.aux_num_regs, air.aux_prog), &jk) == WF_OK;
+        const unsigned blocks = (unsigned)(((ce_rows ? ce_rows : ce) + 127) / 128);
         if (jit) {
             void* args[] = {&p};
-            CK(cudaLaunchKernel((const void*)jk, dim3((unsigned)((ce + 127) / 128)), dim3(128), args, 0, ctx->st));
+            CK(cudaLaunchKernel((const void*)jk, dim3(blocks), dim3(128), args, 0, ctx->st));
         } else if (aw) {
-            generic_constraints_kernel<D, true><<<(unsigned)((ce + 127) / 128), 128, 0, ctx->st>>>(p);
+            generic_constraints_kernel<D, true><<<blocks, 128, 0, ctx->st>>>(p);
         } else {
-            generic_constraints_kernel<D, false><<<(unsigned)((ce + 127) / 128), 128, 0, ctx->st>>>(p);
+            generic_constraints_kernel<D, false><<<blocks, 128, 0, ctx->st>>>(p);
         }
         ctx->launches++;
         CK(cudaGetLastError());
@@ -1204,14 +1231,7 @@ int prove_air(wf_ctx* ctx, const AirHost& air_in, const uint64_t* const* trace_c
     CKI(validate_degrees(ctx, air.all_degrees(), n));
     CKI(validate_assertions(ctx, air.aux_asserts, n, 3, "aux assertion"));
     CKI(validate_assertions(ctx, air.asserts, n, 1, "assertion"));
-    // ---- channel seed: Context::to_elements || pub inputs (channel.rs:57-82, context.rs:119-136) ----
-    // TraceInfo::to_elements (air/src/air/trace_info.rs:209-238)
-    const u64 ti0 = aw ? ((((((u64)c << 8) | 1) << 8) | aw) << 8) | air.nr : ((u64)c << 8);
-    std::vector<u64> seed = {ti0, (u64)n, 1, 0xFFFFFFFFULL, (u64)(n_tr + n_as),
-                             ((u64)o.ext << 24) | ((u64)o.folding << 16) | ((u64)o.rem_max_deg << 8) | o.blowup,
-                             o.grinding, o.num_queries};
-    for (u64 v : air.pub_inputs) seed.push_back(v);
-    Channel<D> ch(h, seed);
+    Channel<D> ch(h, channel_seed(air, n, o));
 
     // ---- 1. trace commitment (lib.rs:497-522) ----
     wf_mat *trace = nullptr, *polys = nullptr, *lde = nullptr, *apolys = nullptr, *alde = nullptr, *comp = nullptr, *cpolys = nullptr,
@@ -1364,15 +1384,7 @@ int prove_air(wf_ctx* ctx, const AirHost& air_in, const uint64_t* const* trace_c
     wf_mark(ctx, "grinding");
     // ---- 8. proof object (lib.rs:464-489; air/src/proof/mod.rs:189-200) ----
     ByteVec w;
-    // Context (context.rs:142-151): TraceInfo, modulus, ProofOptions, num_constraints
-    w.u8_((u8)c); w.u8_((u8)aw); w.u8_((u8)air.nr); w.u8_((u8)log_n); w.u16_(0);
-    w.u8_(8); w.u64_(GL_P);
-    w.u8_((u8)o.num_queries); w.u8_((u8)o.blowup); w.u8_((u8)o.grinding); w.u8_((u8)o.ext); w.u8_((u8)o.folding);
-    w.u8_((u8)o.rem_max_deg); w.u8_((u8)o.batch_c); w.u8_((u8)o.batch_d); w.u8_((u8)o.num_partitions); w.u8_((u8)o.hash_rate);
-    w.usize(n_tr + n_as);
-    w.u8_((u8)pos.size());
-    w.u16_((uint16_t)ch.commitments.v.size());
-    w.bytes(ch.commitments.v.data(), ch.commitments.v.size());
+    write_proof_head(w, air, log_n, o, pos.size(), ch.commitments);
     // every gather of the proof (trace rows, constraint rows, all FRI layers + their Merkle paths)
     // goes through one batch: one index upload, one download, one synchronisation
     GatherBatch gb;
@@ -1537,31 +1549,64 @@ static int shard_tree_finish(ShardCtx& sc, int h, ShardTree& t, Digest* root) {
     return WF_OK;
 }
 
+// Trace columns of rank `rank` of `world` in a sharded proof: the S = ceil(width / 8) segments of the whole trace split as
+// evenly as possible, rank r owning segments [floor(r S / world), floor((r+1) S / world)), i.e. the columns
+// [*first, *first + *count). Narrow traces leave some ranks without a column (*count = 0). When 8 * world divides the width
+// this is the block [r * width / world, (r+1) * width / world) of every rank.
+static bool shard_columns(u32 width, int world, int rank, u32* first, u32* count) {
+    if (width == 0 || width > 255 || world < 2 || (world & (world - 1)) || rank < 0 || rank >= world) return false;
+    const u64 S = (width + 7) / 8;
+    const u32 s0 = (u32)((u64)rank * S / (u64)world), s1 = (u32)((u64)(rank + 1) * S / (u64)world);
+    *first = std::min(8 * s0, width);
+    *count = std::min(8 * s1, width) - *first;
+    return true;
+}
+
+// What a sharded proof needs of its shape; the same on every rank, checked before any device work
+static int sharded_shape_check(wf_ctx* ctx, const AirHost& air, u32 log_n, const Options& o, int G, int r) {
+    if (G < 2 || (G & (G - 1)) || r < 0 || r >= G) return wf_fail(ctx, WF_ERR_INVALID, "world size must be a power of two >= 2");
+    // the FibSmall entry point keeps its contract: every rank passes a block of whole 8-column segments
+    if (air.is_fib && (air.w % (u32)G || (air.w / (u32)G) % 8))
+        return wf_fail(ctx, WF_ERR_UNSUPPORTED, "each rank must own whole 8-column segments (2k / world a multiple of 8)");
+    u32 log_b = 0;
+    while ((1u << log_b) < o.blowup) log_b++;
+    const u32 log_ceb = air.log_ce_blowup();
+    if (log_ceb > log_b) return wf_fail(ctx, WF_ERR_INVALID, "blowup factor too small for the constraint degrees");
+    const size_t rows_per = ((size_t)1 << (log_n + log_b)) / (size_t)G, ce_per = ((size_t)1 << (log_n + log_ceb)) / (size_t)G;
+    if (rows_per < 64 * (size_t)o.blowup || ce_per < 64) return wf_fail(ctx, WF_ERR_UNSUPPORTED, "trace too short to shard over %d ranks", G);
+    return WF_OK;
+}
+
+// One proof of a single-segment AIR sharded over the ranks of `cm` (wf_prove_fib_sharded, wf_prove_air_sharded). The
+// arguments have been checked on every rank alike; this rank passes the columns shard_columns assigns it (none is possible).
 template <int D>
-int prove_fib_sharded(wf_ctx* ctx, const wf_comm* cm, const uint64_t* const* local_cols, const uint64_t* d_local, int mont, u32 k,
-                      u32 log_n, const u64* results, const Options& o, std::vector<u8>& proof_out, double* stats) {
+int prove_sharded(wf_ctx* ctx, const wf_comm* cm, const AirHost& air, const uint64_t* const* local_cols, const uint64_t* d_local, int mont,
+                  u32 log_n, const Options& o, std::vector<u8>& proof_out, double* stats) {
     ShardCtx sc{ctx, cm, cm->world, cm->rank, 0};
     const int G = sc.G, r = sc.r;
+    CKI(sharded_shape_check(ctx, air, log_n, o, G, r));
     while ((1 << sc.logG) < G) sc.logG++;
     const int h = o.hash_id;
     const size_t n = (size_t)1 << log_n;
     u32 log_b = 0;
     while ((1u << log_b) < o.blowup) log_b++;
     const size_t N = n << log_b, b = o.blowup;
-    const u32 c = 2 * k, cl = c / (u32)G, nsl = cl / 8, nsg = c / 8;
-    const size_t rows_per = N / (size_t)G;
-    if (G < 2 || (G & (G - 1)) || r < 0 || r >= G) return wf_fail(ctx, WF_ERR_INVALID, "world size must be a power of two >= 2");
-    if (c % (u32)G || cl % 8) return wf_fail(ctx, WF_ERR_UNSUPPORTED, "each rank must own whole 8-column segments (2k / world a multiple of 8)");
-    const AirHost air = fib_air_host(k, n, results);
+    const u32 c = air.w;
     const u32 kc = air.num_comp_cols(n), log_ceb = air.log_ce_blowup();
-    const size_t ce = n << log_ceb, ce_per = ce / (size_t)G;
-    if (rows_per < 64 * b || ce_per < 64) return wf_fail(ctx, WF_ERR_UNSUPPORTED, "trace too short to shard over %d ranks", G);
+    const size_t rows_per = N / (size_t)G, ce = n << log_ceb, ce_per = ce / (size_t)G;
+    // Column ownership, in segments of the WHOLE trace's width Wg: the row shard, the staging buffer and every rank's local LDE
+    // use that width, so local segment g of rank q is global segment sg0[q] + g and blocks move as whole segment rows
+    const int Wg = seg_width_for(c);
+    const u32 nsg = (c + Wg - 1) / Wg;
+    std::vector<u32> col0(G), ncol(G), sg0(G), nsl(G);
+    for (int q = 0; q < G; q++) {
+        shard_columns(c, G, q, &col0[q], &ncol[q]);
+        sg0[q] = col0[q] / Wg;
+        nsl[q] = (ncol[q] + Wg - 1) / Wg;
+    }
+    const u32 cl = ncol[r];
     const u32 n_tr = (u32)air.degrees.size(), n_as = (u32)air.asserts.size();
-    std::vector<u64> seed = {(u64)c << 8, (u64)n, 1, 0xFFFFFFFFULL, (u64)(n_tr + n_as),
-                             ((u64)o.ext << 24) | ((u64)o.folding << 16) | ((u64)o.rem_max_deg << 8) | o.blowup,
-                             o.grinding, o.num_queries};
-    for (u64 v : air.pub_inputs) seed.push_back(v);
-    Channel<D> ch(h, seed);  // every rank replays the whole transcript
+    Channel<D> ch(h, channel_seed(air, n, o));  // every rank replays the whole transcript
 
     wf_mat *trace = nullptr, *polys = nullptr, *lde = nullptr, *shard = nullptr, *comp_l = nullptr, *comp = nullptr, *cpolys = nullptr,
            *clde = nullptr, *deep = nullptr, *fri_in = nullptr, *tstage = nullptr;
@@ -1584,8 +1629,9 @@ int prove_fib_sharded(wf_ctx* ctx, const wf_comm* cm, const uint64_t* const* loc
     //         block per segment: its exchange runs on the communicator's stream while coset k + 1 is being extended ----
     wf_mark(ctx, "start");
     const size_t nj = n / (size_t)G;   // points of one coset inside one rank's row range
-    CKI(wf_mat_alloc(ctx, rows_per + b, c, &shard));
-    shard->m.rows = rows_per;  // seg_stride stays (rows_per + b) * 8: rows [rows_per, rows_per + b) are the halo
+    const size_t blk = nj * (size_t)Wg * 8;   // bytes of one (segment, coset, row range) block
+    CKI(wf_mat_alloc(ctx, rows_per + b, c, &shard));   // segment width Wg
+    shard->m.rows = rows_per;  // seg_stride stays (rows_per + b) * Wg: rows [rows_per, rows_per + b) are the halo
     const size_t sstride = shard->m.seg_stride;
     // Transport 1 — the exchange fused into the LDE: every rank maps the others' row shards (CUDA IPC) and the last
     // pass of every coset's transform writes each row straight to its owner (and the first rows of a range also into the halo
@@ -1596,25 +1642,27 @@ int prove_fib_sharded(wf_ctx* ctx, const wf_comm* cm, const uint64_t* const* loc
     while (((size_t)1 << log_nj) < nj) log_nj++;
     // (measured at 2 GPUs, cfg3: the remote 64-byte stores stall the pass by about what the transfer costs — 37.4 ms LDE + 0.6 ms
     // exposed against 30.3 + 5.6 with copy-engine pushes and 28.1 + 8.1 with a blocking NCCL all-to-all — so the fused form is
-    // opt-in, WF_FUSED_SCATTER=1, and the copy-engine push below is the default)
+    // opt-in, WF_FUSED_SCATTER=1, and the copy-engine push below is the default). The fused form places rank r's segments at
+    // one offset per rank: it needs every rank to own the same number of whole 8-column segments; other splits take the push.
     const char* fused_env = getenv("WF_FUSED_SCATTER");
-    const bool scat = fused_env && atoi(fused_env) != 0 && G <= 8 && log_n <= 22 && sc.map_peers(shard->m.base, peer_shard) == WF_OK;
+    const bool even = c % (8 * (u32)G) == 0;
+    const bool scat = fused_env && atoi(fused_env) != 0 && even && G <= 8 && log_n <= 22 && sc.map_peers(shard->m.base, peer_shard) == WF_OK;
     bool push = false;
     if (scat) {
         LdeScatter sct;
         for (int q = 0; q < 8; q++) sct.peer[q] = q < G ? (u64*)peer_shard[q] : nullptr;
-        sct.seg_stride = sstride; sct.seg0 = (u32)r * nsl; sct.log_nj = log_nj; sct.world = (u32)G;
+        sct.seg_stride = sstride; sct.seg0 = sg0[r]; sct.log_nj = log_nj; sct.world = (u32)G;
         CKI(wf_trace_lde_cosetwise(ctx, local_cols, d_local, cl, n, mont, log_b, &polys, nullptr, false, nullptr, &sct));
         wf_mark(ctx, "trace_lde");
         CK(cudaStreamSynchronize(ctx->st));   // my stores have landed; everybody's have when every rank says so
         CKI(sc.host_barrier());
         sc.ncoll += 1;
-        sc.bytes_overlapped += (double)(G - 1) * nsl * (double)rows_per * 64;
+        sc.bytes_overlapped += (double)(G - 1) * nsl[r] * (double)rows_per * Wg * 8;
         push = true;
     } else {
-    wf_mat*& stage = tstage;           // what arrives: [global segment][coset][nj][8]
-    CKI(wf_mat_alloc_w(ctx, N, cl, 8, &lde));          // mine, coset-major: [local segment][coset][n][8]
-    CKI(wf_mat_alloc_w(ctx, rows_per, c, 8, &stage));
+    wf_mat*& stage = tstage;           // what arrives: [global segment][coset][nj][Wg]
+    if (cl) CKI(wf_mat_alloc_w(ctx, N, cl, Wg, &lde));   // mine, coset-major: [local segment][coset][n][Wg]
+    CKI(wf_mat_alloc_w(ctx, rows_per, c, Wg, &stage));
     // Preferred transport: every rank maps the others' `stage` buffers (CUDA IPC) and PUSHES its blocks there with peer copies
     // on side streams — copy engines over NVLink, no SM taken from the NTT kernels they overlap (NCCL send/recv kernels on a
     // side stream were measured: they slow the LDE down by as much as they hide). Fallback: the communicator's exchange.
@@ -1624,44 +1672,44 @@ int prove_fib_sharded(wf_ctx* ctx, const wf_comm* cm, const uint64_t* const* loc
         for (int i = 0; i < 4; i++) if (!ctx->push_st[i]) CK(cudaStreamCreateWithFlags(&ctx->push_st[i], cudaStreamNonBlocking));
         for (int i = 0; i < 16; i++) if (!ctx->push_ev[i]) CK(cudaEventCreateWithFlags(&ctx->push_ev[i], cudaEventDisableTiming));
     }
+    // block of my local segment sg, coset k, that belongs to rank q's rows; the block's place in a stage buffer
+    auto my_block = [&](u32 sg, u32 k, int q) { return lde->m.base + (size_t)sg * lde->m.seg_stride + ((size_t)k * n + (size_t)q * nj) * Wg; };
+    auto stage_block = [&](u64* base, u32 gseg, u32 k) { return base + (size_t)gseg * stage->m.seg_stride + (size_t)k * nj * Wg; };
     const std::function<int(u32)> after_coset = [&](u32 k) -> int {   // coset k of every local column is enqueued: ship it
         if (push) {
             cudaEvent_t ev = ctx->push_ev[k % 16];
             CK(cudaEventRecord(ev, ctx->st));
-            for (int dq = 1; dq < G; dq++) {             // start with the next rank: no two ranks hit the same peer first
+            for (int dq = 1; dq < G && nsl[r]; dq++) {   // start with the next rank: no two ranks hit the same peer first
                 const int q = (r + dq) % G;
                 cudaStream_t ps = ctx->push_st[dq % 4];
                 CK(cudaStreamWaitEvent(ps, ev, 0));
-                for (u32 sg = 0; sg < nsl; sg++) {
-                    const u64* src = lde->m.base + (size_t)sg * lde->m.seg_stride + ((size_t)k * n + (size_t)q * nj) * 8;
-                    u64* dst = (u64*)peer_stage[q] + ((size_t)r * nsl + sg) * stage->m.seg_stride + (size_t)k * nj * 8;
-                    CK(cudaMemcpyAsync(dst, src, nj * 64, cudaMemcpyDeviceToDevice, ps));
-                }
+                for (u32 sg = 0; sg < nsl[r]; sg++)
+                    CK(cudaMemcpyAsync(stage_block((u64*)peer_stage[q], sg0[r] + sg, k), my_block(sg, k, q), blk, cudaMemcpyDeviceToDevice, ps));
             }
-            for (u32 sg = 0; sg < nsl; sg++) {
-                const u64* src = lde->m.base + (size_t)sg * lde->m.seg_stride + ((size_t)k * n + (size_t)r * nj) * 8;
-                CK(cudaMemcpyAsync(stage->m.base + ((size_t)r * nsl + sg) * stage->m.seg_stride + (size_t)k * nj * 8, src, nj * 64,
-                                   cudaMemcpyDeviceToDevice, ctx->st));
-            }
-            sc.bytes_overlapped += (double)(G - 1) * nsl * nj * 64;
+            for (u32 sg = 0; sg < nsl[r]; sg++)
+                CK(cudaMemcpyAsync(stage_block(stage->m.base, sg0[r] + sg, k), my_block(sg, k, r), blk, cudaMemcpyDeviceToDevice, ctx->st));
+            sc.bytes_overlapped += (double)(G - 1) * nsl[r] * blk;
             return WF_OK;
         }
+        // pairwise order: sender r -> q lists my segments ascending; receiver r <- q lists q's segments ascending
         std::vector<int> sp, rp;
         std::vector<const void*> sv;
         std::vector<void*> rv;
-        for (u32 sg = 0; sg < nsl; sg++)
+        for (u32 sg = 0; sg < nsl[r]; sg++)
             for (int q = 0; q < G; q++) {
-                const u64* src = lde->m.base + (size_t)sg * lde->m.seg_stride + ((size_t)k * n + (size_t)q * nj) * 8;
-                u64* dst = stage->m.base + ((size_t)q * nsl + sg) * stage->m.seg_stride + (size_t)k * nj * 8;   // q = the SOURCE rank here
-                if (q == r) CK(cudaMemcpyAsync(dst, src, nj * 64, cudaMemcpyDeviceToDevice, ctx->st));
-                else { sp.push_back(q); sv.push_back(src); rp.push_back(q); rv.push_back(dst); }
+                if (q == r) CK(cudaMemcpyAsync(stage_block(stage->m.base, sg0[r] + sg, k), my_block(sg, k, r), blk, cudaMemcpyDeviceToDevice, ctx->st));
+                else { sp.push_back(q); sv.push_back(my_block(sg, k, q)); }
             }
+        for (int q = 0; q < G; q++)
+            for (u32 sg = 0; q != r && sg < nsl[q]; sg++) { rp.push_back(q); rv.push_back(stage_block(stage->m.base, sg0[q] + sg, k)); }
         CKI(sc.fork());
-        return sc.exchange(sp, sv, rp, rv, nj * 64);
+        return sc.exchange(sp, sv, rp, rv, blk);
     };
     // (upload ->) layout -> interpolate -> extend, pipelined per column chunk for host columns; the cosets of the last chunk
-    // are extended one by one and after_coset(k) ships coset k while coset k + 1 is computed
-    CKI(wf_trace_lde_cosetwise(ctx, local_cols, d_local, cl, n, mont, log_b, &polys, &lde, true, &after_coset, nullptr));
+    // are extended one by one and after_coset(k) ships coset k while coset k + 1 is computed. A rank without columns only
+    // takes part in the exchanges.
+    if (cl) CKI(wf_trace_lde_cosetwise(ctx, local_cols, d_local, cl, n, mont, log_b, &polys, &lde, true, &after_coset, nullptr));
+    else for (u32 k = 0; k < (u32)b; k++) CKI(after_coset(k));
     wf_mark(ctx, "trace_lde");
     if (push) {
         // my pushes have landed when my side streams drain; everybody's have when every rank says so
@@ -1673,7 +1721,7 @@ int prove_fib_sharded(wf_ctx* ctx, const wf_comm* cm, const uint64_t* const* loc
     }
     {   // coset-major -> natural order (row = b j + k) of my row range, every segment
         SegMatrix dstv = shard->m;
-        dim3 grid((unsigned)((rows_per * 8 + 255) / 256), nsg);
+        dim3 grid((unsigned)((rows_per * Wg + 255) / 256), nsg);
         coset_interleave_kernel<<<grid, 256, 0, ctx->st>>>(stage->m, dstv, nj, (u32)b);
         ctx->launches++;
         CK(cudaGetLastError());
@@ -1682,12 +1730,12 @@ int prove_fib_sharded(wf_ctx* ctx, const wf_comm* cm, const uint64_t* const* loc
     scope.drop(stage);
     {   // halo: the first `blowup` rows of every segment of rank (r + 1) mod G
         void *pk, *pk2;
-        const size_t hb = b * 64;
+        const size_t hb = b * Wg * 8;
         CKI(wf_dev_alloc(ctx, hb * nsg, &pk));
         CKI(wf_dev_alloc(ctx, hb * nsg, &pk2));
         CK(cudaMemcpy2DAsync(pk, hb, shard->m.base, sstride * 8, hb, nsg, cudaMemcpyDeviceToDevice, ctx->st));
         CKI(sc.exchange({(r + G - 1) % G}, {pk}, {(r + 1) % G}, {pk2}, hb * nsg));
-        CK(cudaMemcpy2DAsync(shard->m.base + rows_per * 8, sstride * 8, pk2, hb, hb, nsg, cudaMemcpyDeviceToDevice, ctx->st));
+        CK(cudaMemcpy2DAsync(shard->m.base + rows_per * Wg, sstride * 8, pk2, hb, hb, nsg, cudaMemcpyDeviceToDevice, ctx->st));
         wf_dev_free(ctx, pk);
         wf_dev_free(ctx, pk2);
     }
@@ -1771,19 +1819,26 @@ int prove_fib_sharded(wf_ctx* ctx, const wf_comm* cm, const uint64_t* const* loc
     CKI(shard_tree_finish(sc, h, ctree, &root));
     wf_mark(ctx, "composition_commit");
     ch.commit(root.b);
-    // ---- 6. out-of-domain frames: my columns' polynomials, all-gathered; composition columns are replicated ----
+    // ---- 6. out-of-domain frames: my columns' polynomials, all-gathered (every rank's part padded to the largest rank's
+    //         column count: the gather takes equal sizes); composition columns are replicated ----
     GlExt<D> z = ch.draw();
     GlExt<D> zg = ext_mul_base(z, gl_root_of_unity(log_n));
-    std::vector<std::vector<GlExt<D>>> ood;
-    CKI(ood_eval<D>(ctx, {polys, cpolys}, z, zg, ood));
+    std::vector<std::vector<GlExt<D>>> ood;   // [0], [1]: composition columns at z, zg; [2], [3]: my trace columns
+    std::vector<const wf_mat*> om = {cpolys};
+    if (cl) om.push_back(polys);
+    CKI(ood_eval<D>(ctx, om, z, zg, ood));
     std::vector<GlExt<D>> t_cur(c), t_nxt(c);
     {
-        std::vector<u64> mine((size_t)cl * 2 * D), all((size_t)c * 2 * D);
+        const u32 cmax = *std::max_element(ncol.begin(), ncol.end());
+        std::vector<u64> mine((size_t)cmax * 2 * D, 0), all((size_t)G * cmax * 2 * D);
         for (u32 j = 0; j < cl; j++)
-            for (int q = 0; q < D; q++) { mine[((size_t)j * 2) * D + q] = ood[0][j].v[q]; mine[((size_t)j * 2 + 1) * D + q] = ood[1][j].v[q]; }
+            for (int q = 0; q < D; q++) { mine[((size_t)j * 2) * D + q] = ood[2][j].v[q]; mine[((size_t)j * 2 + 1) * D + q] = ood[3][j].v[q]; }
         CKI(sc.gather_host(mine.data(), all.data(), mine.size() * 8));
-        for (u32 j = 0; j < c; j++)
-            for (int q = 0; q < D; q++) { t_cur[j].v[q] = all[((size_t)j * 2) * D + q]; t_nxt[j].v[q] = all[((size_t)j * 2 + 1) * D + q]; }
+        for (int rq = 0; rq < G; rq++)
+            for (u32 j = 0; j < ncol[rq]; j++) {
+                const u64* e = &all[((size_t)rq * cmax + j) * 2 * D];
+                for (int q = 0; q < D; q++) { t_cur[col0[rq] + j].v[q] = e[q]; t_nxt[col0[rq] + j].v[q] = e[D + q]; }
+            }
     }
     auto combine = [&](const std::vector<GlExt<D>>& comp_evals) {  // H_j(z) from its base-component columns
         std::vector<GlExt<D>> rr(comp_evals.size() / D);
@@ -1798,7 +1853,7 @@ int prove_fib_sharded(wf_ctx* ctx, const wf_comm* cm, const uint64_t* const* loc
         }
         return rr;
     };
-    std::vector<GlExt<D>> q_cur = combine(ood[2]), q_nxt = combine(ood[3]);
+    std::vector<GlExt<D>> q_cur = combine(ood[0]), q_nxt = combine(ood[1]);
     ByteVec ood_t, ood_q;
     ood_t.u8_(2); write_elems<D>(ood_t, t_cur); write_elems<D>(ood_t, t_nxt);
     ood_q.u8_(2); write_elems<D>(ood_q, q_cur); write_elems<D>(ood_q, q_nxt);
@@ -1896,14 +1951,7 @@ int prove_fib_sharded(wf_ctx* ctx, const wf_comm* cm, const uint64_t* const* loc
     wf_mark(ctx, "grinding");
     // ---- 10. proof object: every rank queues the same gathers, contributes what it holds, the words are summed ----
     ByteVec w;
-    w.u8_((u8)c); w.u8_(0); w.u8_(0); w.u8_((u8)log_n); w.u16_(0);
-    w.u8_(8); w.u64_(GL_P);
-    w.u8_((u8)o.num_queries); w.u8_((u8)o.blowup); w.u8_((u8)o.grinding); w.u8_((u8)o.ext); w.u8_((u8)o.folding);
-    w.u8_((u8)o.rem_max_deg); w.u8_((u8)o.batch_c); w.u8_((u8)o.batch_d); w.u8_((u8)o.num_partitions); w.u8_((u8)o.hash_rate);
-    w.usize(n_tr + n_as);
-    w.u8_((u8)pos.size());
-    w.u16_((uint16_t)ch.commitments.v.size());
-    w.bytes(ch.commitments.v.data(), ch.commitments.v.size());
+    write_proof_head(w, air, log_n, o, pos.size(), ch.commitments);
     GatherBatch gb;
     gb.comm = cm;
     const u64 NONE = ~(u64)0;
@@ -2243,6 +2291,22 @@ extern "C" int wf_deep_compose(wf_ctx* ctx, uint32_t ext, const wf_mat* main_lde
     }
 }
 
+static int prove_sharded_dispatch(wf_ctx* ctx, const wf_comm* comm, const AirHost& air, const uint64_t* const* local_cols,
+                                  const uint64_t* d_local, int mont, uint32_t log_n, const Options& o, uint8_t* proof, size_t* proof_len,
+                                  double* stats) {
+    std::vector<u8> out;
+    int r;
+    switch (o.ext) {
+        case 1: r = prove_sharded<1>(ctx, comm, air, local_cols, d_local, mont, log_n, o, out, stats); break;
+        case 2: r = prove_sharded<2>(ctx, comm, air, local_cols, d_local, mont, log_n, o, out, stats); break;
+        default: r = prove_sharded<3>(ctx, comm, air, local_cols, d_local, mont, log_n, o, out, stats); break;
+    }
+    if (r != WF_OK) return r;
+    if (out.size() > *proof_len) return wf_fail(ctx, WF_ERR_INVALID, "proof buffer too small (%zu needed)", out.size());
+    memcpy(proof, out.data(), out.size());
+    *proof_len = out.size();
+    return WF_OK;
+}
 extern "C" int wf_prove_fib_sharded(wf_ctx* ctx, const wf_comm* comm, const uint64_t* const* local_cols, const uint64_t* d_local, int mont,
                                     uint32_t k, uint32_t log_n, const uint64_t* results, const uint32_t* opts, uint8_t* proof,
                                     size_t* proof_len, double* stats) {
@@ -2251,18 +2315,61 @@ extern "C" int wf_prove_fib_sharded(wf_ctx* ctx, const wf_comm* comm, const uint
         return wf_fail(ctx, WF_ERR_INVALID, "bad arguments");
     Options o;
     CKI(parse_options(ctx, opts, o));
-    std::vector<u8> out;
-    int r;
-    switch (o.ext) {
-        case 1: r = prove_fib_sharded<1>(ctx, comm, local_cols, d_local, mont, k, log_n, results, o, out, stats); break;
-        case 2: r = prove_fib_sharded<2>(ctx, comm, local_cols, d_local, mont, k, log_n, results, o, out, stats); break;
-        default: r = prove_fib_sharded<3>(ctx, comm, local_cols, d_local, mont, k, log_n, results, o, out, stats); break;
+    const AirHost air = fib_air_host(k, (size_t)1 << log_n, results);
+    return prove_sharded_dispatch(ctx, comm, air, local_cols, d_local, mont, log_n, o, proof, proof_len, stats);
+}
+extern "C" int wf_host_shard_columns(uint32_t width, int world, int rank, uint32_t* first, uint32_t* count) {
+    if (!first || !count) return WF_ERR_INVALID;
+    return shard_columns(width, world, rank, first, count) ? WF_OK : WF_ERR_INVALID;
+}
+// A sharded proof must not start unless every rank can go through with it: a rank that refused would otherwise leave the
+// others waiting in a collective. So each rank checks its own arguments (no device work), hashes what must be equal on
+// every rank, and one all-gather of (status, hash) decides for all of them.
+extern "C" int wf_prove_air_sharded(wf_ctx* ctx, const wf_comm* comm, const uint64_t* air_desc, size_t air_desc_len,
+                                    const uint64_t* const* local_cols, const uint64_t* d_local, int mont, uint32_t log_n,
+                                    const uint32_t* opts, uint8_t* proof, size_t* proof_len, double* stats) {
+    if (!ctx || !comm || !comm->exchange || !comm->all_gather_host || !comm->all_reduce_sum || comm->world < 1 || comm->rank < 0 ||
+        comm->rank >= comm->world)
+        return wf_fail(ctx, WF_ERR_INVALID, "bad arguments");   // no communicator to agree over
+    const int G = comm->world, r = comm->rank;
+    Options o;
+    AirHost air;
+    auto own_checks = [&]() -> int {
+        if (!air_desc || !opts || !proof || !proof_len || log_n < 3 || log_n > 32) return wf_fail(ctx, WF_ERR_INVALID, "bad arguments");
+        CKI(parse_options(ctx, opts, o));
+        if (!parse_air_host(air_desc, air_desc_len, air)) return wf_fail(ctx, WF_ERR_INVALID, "malformed AIR description");
+        if (air.aw) return wf_fail(ctx, WF_ERR_UNSUPPORTED, "sharded proofs cover single-segment AIRs (this description has an auxiliary segment)");
+        CKI(sharded_shape_check(ctx, air, log_n, o, G, r));
+        const size_t n = (size_t)1 << log_n;
+        for (auto& col : air.periodic) if (col.size() > n) return wf_fail(ctx, WF_ERR_INVALID, "periodic column longer than the trace");
+        CKI(validate_degrees(ctx, air.all_degrees(), n));
+        CKI(validate_assertions(ctx, air.asserts, n, 1, "assertion"));
+        u32 first = 0, count = 0;
+        shard_columns(air.w, G, r, &first, &count);
+        if (count && !local_cols && !d_local) return wf_fail(ctx, WF_ERR_INVALID, "rank %d owns columns [%u, %u) but passed none", r, first, first + count);
+        if (!count && (local_cols || d_local)) return wf_fail(ctx, WF_ERR_INVALID, "rank %d owns no column but passed some", r);
+        return WF_OK;
+    };
+    const int mine = own_checks();
+    u64 hsh = 0xcbf29ce484222325ULL;   // FNV-1a over the description, log_n, the options and the world size
+    auto mix = [&](u64 v) { for (int i = 0; i < 8; i++) { hsh ^= (v >> (8 * i)) & 0xff; hsh *= 0x100000001b3ULL; } };
+    mix(air_desc ? air_desc_len : ~(u64)0);
+    for (size_t i = 0; air_desc && i < air_desc_len; i++) mix(air_desc[i]);
+    mix(log_n);
+    for (int i = 0; i < 9; i++) mix(opts ? opts[i] : ~(u64)0);
+    mix((u64)G);
+    struct Vote { int32_t status, pad; u64 hash; } v{mine, 0, hsh};
+    std::vector<Vote> all(G);
+    if (comm->all_gather_host(comm->user, &v, all.data(), sizeof(Vote)) != 0) return wf_fail(ctx, WF_ERR_STATE, "all_gather_host callback failed");
+    for (int q = 0; q < G; q++) {   // the lowest refusing rank's status, on every rank
+        if (all[q].status == WF_OK) continue;
+        if (q == r) return mine;
+        const std::string own = mine == WF_OK ? std::string() : "; this rank: " + ctx->err;
+        return wf_fail(ctx, all[q].status, "rank %d refused the sharded proof%s", q, own.c_str());
     }
-    if (r != WF_OK) return r;
-    if (out.size() > *proof_len) return wf_fail(ctx, WF_ERR_INVALID, "proof buffer too small (%zu needed)", out.size());
-    memcpy(proof, out.data(), out.size());
-    *proof_len = out.size();
-    return WF_OK;
+    for (int q = 0; q < G; q++)
+        if (all[q].hash != hsh) return wf_fail(ctx, WF_ERR_INVALID, "ranks %d and %d were given different AIR descriptions, trace lengths, options or world sizes", r, q);
+    return prove_sharded_dispatch(ctx, comm, air, local_cols, d_local, mont, log_n, o, proof, proof_len, stats);
 }
 extern "C" int wf_prove_fib(wf_ctx* ctx, const uint64_t* const* trace_cols, int mont, uint32_t k, uint32_t log_n,
                             const uint64_t* results, const uint32_t* opts, uint8_t* proof, size_t* proof_len) {

@@ -129,7 +129,8 @@ def sharded_trace_commit(backend, hash_id, local_cols, ncols_total, log_n, log_b
 
 
 # --------------------------------------------------------------------------------------------------
-# One proof sharded over the ranks of a torch.distributed group (wf_prove_fib_sharded, include/winterfell_b200.h).
+# One proof sharded over the ranks of a torch.distributed group (wf_prove_fib_sharded, wf_prove_air_sharded,
+# include/winterfell_b200.h).
 # The library does all arithmetic and orchestration; this module only supplies the three collectives of `wf_comm`.
 # --------------------------------------------------------------------------------------------------
 import ctypes as C
@@ -284,6 +285,46 @@ def prove_fib_sharded(ctx, comm, local_trace, k, log_n, results, opts, out_buf=N
                                      o_.ctypes.data_as(C.POINTER(C.c_uint32)), buf.ctypes.data_as(wf.u8p), C.byref(ln), st))
     if comm.error is not None:
         raise comm.error
+    if stats is not None:
+        stats.update({"bytes_sent": st[0], "exchange_ms": st[1], "collectives": st[2], "small_collective_ms": st[3], "sharded_fri_layers": st[4],
+                      "bytes_overlapped": st[5], "peer_push": st[6]})
+    return buf[: ln.value].tobytes()
+
+
+def prove_air_sharded(ctx, comm, desc, local_trace, log_n, opts, mont=False, device_ptr=None, stats=None, out_buf=None):
+    """One proof of a single-segment AIR description (as Context.prove_air) over comm.world GPUs. local_trace: this rank's
+    columns (wf.shard_columns(width, world, rank)) as a [count, n] uint64 host array, or device_ptr = raw pointer to the same
+    block column-major in HBM; a rank that owns no column passes an empty array or None. desc, log_n and opts are the whole
+    proof's. Returns the proof bytes (identical on every rank). Every rank raises when any rank refuses the arguments."""
+    L = wf.lib()
+    d_ = np.ascontiguousarray(desc, dtype=np.uint64)
+    o_ = np.ascontiguousarray(opts, dtype=np.uint32)
+    buf = out_buf if out_buf is not None else np.zeros(1 << 23, dtype=np.uint8)
+    ln = C.c_size_t(buf.size)
+    st = (C.c_double * 8)()
+    ptrs, dptr, wrong = None, None, None
+    if device_ptr is not None:
+        dptr = C.c_void_p(device_ptr)
+    elif local_trace is not None and len(local_trace):
+        a = np.ascontiguousarray(local_trace, dtype=np.uint64)
+        ptrs = (wf.u64p * a.shape[0])(*[a[j].ctypes.data_as(wf.u64p) for j in range(a.shape[0])])
+        try:
+            _, count = wf.shard_columns(int(d_[0]) if d_.size else 0, comm.world, comm.rank)
+        except wf.WfError:   # no ownership to compare against: the library refuses the description or the world size itself
+            count = a.shape[0]
+        if a.shape[0] != count or a.shape[1] != 1 << log_n:
+            # the library cannot see the length of a column list: this rank passes no columns, which the library refuses for a
+            # rank that owns some (and columns, which it refuses for one that owns none), so the refusal goes through its
+            # agreement step and every rank returns the error instead of waiting on this one
+            wrong = f"rank {comm.rank} passed a [{a.shape[0]}, {a.shape[1]}] block, owns {count} columns of {1 << log_n} rows"
+            ptrs = None if count else ptrs
+    r = L.wf_prove_air_sharded(ctx.h, C.byref(comm.struct), d_.ctypes.data_as(wf.u64p), d_.size, ptrs, dptr, int(mont), log_n,
+                               o_.ctypes.data_as(C.POINTER(C.c_uint32)), buf.ctypes.data_as(wf.u8p), C.byref(ln), st)
+    if comm.error is not None:
+        raise comm.error
+    if r != wf.WF_OK and wrong:
+        raise wf.WfError(f"error {r}: {wrong}")
+    ctx.check(r)
     if stats is not None:
         stats.update({"bytes_sent": st[0], "exchange_ms": st[1], "collectives": st[2], "small_collective_ms": st[3], "sharded_fri_layers": st[4],
                       "bytes_overlapped": st[5], "peer_push": st[6]})
