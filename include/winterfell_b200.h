@@ -329,6 +329,31 @@ int wf_host_shard_columns(uint32_t width, int world, int rank, uint32_t* first, 
 int wf_prove_air_sharded(wf_ctx* ctx, const wf_comm* comm, const uint64_t* air_desc, size_t air_desc_len,
                          const uint64_t* const* local_cols, const uint64_t* d_local, int mont, uint32_t log_n,
                          const uint32_t* opts, uint8_t* proof, size_t* proof_len, double* stats);
+/* Aux columns this rank builds: E columns [first_col, first_col + num_cols) of the aux segment, written to
+ * aux_out = [num_cols][n][d] words (one Vec<E> per column, as wf_aux_builder_fn). Returns 0 on success. */
+typedef int (*wf_aux_shard_builder_fn)(void* user, const uint64_t* rand_elements, uint32_t first_col, uint32_t num_cols,
+                                       uint64_t* aux_out);
+/* wf_prove_air_aux / wf_prove_air_aux_dyn (description WITH an aux segment) sharded over comm->world GPUs; every rank returns
+ * the same bytes, equal to those one-GPU calls' for the same description, trace, builder and options. The main trace is
+ * passed as in wf_prove_air_sharded.
+ * Aux ownership: the aux segment is aw * d BASE columns (component q of E column j is base column j d + q) and rank r owns
+ * base columns [first, first + count) = wf_host_shard_columns(aw * d, world, r). After the main commitment every rank draws
+ * the same random elements (Montgomery form under `mont`, as wf_prove_air_aux) and calls aux_builder ONCE with the E columns
+ * covering its base columns: first_col = first / d, num_cols = ceil((first + count) / d) - first_col; a rank that owns no aux
+ * base column is not called. With d > 1 one E column can straddle two ranks: both build it and each keeps its own
+ * components, so the builder must be deterministic. aux_assertions (NULL: the description's static aux assertions) is
+ * called on EVERY rank as in wf_prove_air_aux_dyn; it must return the same values everywhere (Air::get_aux_assertions
+ * depends only on public inputs and random elements).
+ * Agreement: before any device work as wf_prove_air_sharded, plus WF_ERR_INVALID for a description without an aux segment,
+ * a NULL aux_builder, or aux assertions that do not validate. After the callbacks the ranks all-gather (callback status,
+ * hash of the aux assertion values): if a callback failed on any rank, every rank returns the lowest failing rank's status;
+ * if the values differ, every rank returns WF_ERR_INVALID. stats: as wf_prove_air_sharded ([6] describes the main trace's
+ * transport), and [7] = milliseconds this rank spent inside aux_builder and aux_assertions. */
+int wf_prove_air_aux_sharded(wf_ctx* ctx, const wf_comm* comm, const uint64_t* air_desc, size_t air_desc_len,
+                             const uint64_t* const* local_cols, const uint64_t* d_local, int mont, uint32_t log_n,
+                             const uint32_t* opts, wf_aux_shard_builder_fn aux_builder,
+                             wf_aux_assertions_fn aux_assertions /* NULL: static aux assertions */, void* aux_user,
+                             uint8_t* proof, size_t* proof_len, double* stats);
 
 /* ---- constraint kernels compiled per AIR ---------------------------------------------------------------------------
  * wf_eval_constraints / wf_prove_air[_aux] evaluate the AIR's transition programs with a kernel compiled at run time for that

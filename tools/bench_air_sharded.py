@@ -1,12 +1,15 @@
-"""Strong scaling of wf_prove_air_sharded: one proof of an AIR description over N GPUs of a node (NCCL), against the one-GPU
-proof. Start with torchrun, one process per GPU:
+"""Strong scaling of wf_prove_air_sharded / wf_prove_air_aux_sharded: one proof of an AIR description over N GPUs of a node
+(NCCL), against the one-GPU proof. Start with torchrun, one process per GPU:
 
-    torchrun --nproc-per-node=N tools/bench_air_sharded.py [--cases fib16,rescue6] [--steps 5] [--warmup 2] [--out FILE]
+    torchrun --nproc-per-node=N tools/bench_air_sharded.py [--cases fib16,rescue6,rap] [--steps 5] [--warmup 2] [--out FILE]
 
 Cases: `fib16` = FibSmall x 16 (32 columns) at 2^22 rows described generically (the bytecode evaluator / its NVRTC kernel),
 next to wf_prove_fib_sharded (the specialised kernel) on the same trace where its whole-segment rule allows; `rescue6` =
-rescue_like(6) at 2^20 rows (degree 7), the widest Rescue-like AIR a description can express. N = 1 times wf_prove_air on one
-GPU (host columns: the one-GPU AIR entry point takes no device trace) and wf_prove_fib_dev. Per case rank 0 prints one JSON
+rescue_like(6) at 2^20 rows (degree 7), the widest Rescue-like AIR a description can express; `rap` (opt-in, not in the default
+list) = perm_rap_lanes(3) at 2^20 rows, a two-segment AIR whose aux columns a host callback builds (each rank builds only the
+lanes covering its aux columns; the line's "callback_ms" is the time spent in the callbacks per proof, max over ranks). N = 1
+times wf_prove_air (wf_prove_air_aux for `rap`) on one GPU (host columns: the one-GPU AIR entry points take no device trace)
+and wf_prove_fib_dev. Per case rank 0 prints one JSON
 line: ms per proof (CUDA events on the context stream, max over ranks of the per-rank mean, 256 MiB L2 flush before every
 step), the library's stage times and stats, byte identity against the one-GPU proof (checked once, before timing), and the
 card's name, power limit and SM clock read in the same run. Traces are built once and cached in a temporary directory."""
@@ -27,6 +30,7 @@ import torch
 import torch.distributed as dist
 
 import airs
+import airs_aux
 import winterfell_b200 as wf
 from oracle import oracle as O
 from winterfell_b200 import dist as wd
@@ -48,6 +52,10 @@ def fib_desc(k, n, results):
 
 
 def load_case(name, cache):
+    if name == "rap":   # returns the aux builder in place of FibSmall results
+        log_n = 20
+        desc, trace, builder = airs_aux.perm_rap_lanes(1 << log_n)
+        return log_n, desc, trace, builder
     if name == "fib16":
         log_n = 22
         trace, results = wf.build_fib_trace(16, 1 << log_n)
@@ -120,7 +128,27 @@ def main():
         opts = O.make_opts(**OPTS)
         width = trace.shape[0]
         variants = {}
-        if world == 1:
+        cb_ms = []   # one-GPU `rap`: time inside the aux builder, per proof
+        if name == "rap":
+            builder, results = results, None
+            aw, nr, _ = wf.aux_shape(desc)
+
+            def one_gpu_builder(rand):
+                t0 = time.perf_counter()
+                aux = builder(rand)
+                cb_ms.append((time.perf_counter() - t0) * 1e3)
+                return aux
+        if name == "rap" and world == 1:
+            pinned = torch.from_numpy(trace.view(np.int64)).pin_memory().numpy().view(np.uint64)
+            variants["air_aux"] = (lambda: ctx.prove_air_aux(desc, pinned, opts, one_gpu_builder, aw, nr), "host columns (pinned)")
+        elif name == "rap":
+            first, count = wf.shard_columns(width, world, rank)
+            local = torch.from_numpy(np.ascontiguousarray(trace[first:first + count]).view(np.int64)).cuda()
+            ptr = local.data_ptr() if count else None
+            stats = {}
+            variants["air_aux"] = (lambda: wd.prove_air_aux_sharded(ctx, comm, desc, None, log_n, opts, builder.columns, device_ptr=ptr,
+                                                                    stats=stats, out_buf=out_buf), "resident main columns")
+        elif world == 1:
             pinned = torch.from_numpy(trace.view(np.int64)).pin_memory().numpy().view(np.uint64)
             variants["air"] = (lambda: ctx.prove_air(desc, pinned, opts), "host columns (pinned)")
             if results is not None:
@@ -138,7 +166,12 @@ def main():
                 variants["fib_specialised"] = (lambda: wd.prove_fib_sharded(ctx, comm, None, width // 2, log_n, results, opts, out_buf=out_buf,
                                                                             device_ptr=local.data_ptr(), stats=stats), "resident")
         with torch.cuda.stream(stream):
-            want = ctx.prove_air(desc, trace, opts) if rank == 0 else None   # the one-GPU proof, untimed
+            if rank != 0:
+                want = None
+            elif name == "rap":
+                want = ctx.prove_air_aux(desc, trace, opts, builder, aw, nr)
+            else:
+                want = ctx.prove_air(desc, trace, opts)   # the one-GPU proof, untimed
             for vname, (fn, inp) in variants.items():
                 t0 = time.perf_counter()
                 first_proof = fn()
@@ -147,12 +180,20 @@ def main():
                     fn()
                 identical = (first_proof == want) if rank == 0 else None
                 before = card(local_rank)
+                cb_ms.clear()
                 ms, per = timed(fn)
                 after = card(local_rank)
+                callback = None
+                if name == "rap":   # this rank's callback time per proof (the last timed step), max over the ranks
+                    mine = cb_ms[-1] if world == 1 else stats["callback_ms"]
+                    t = torch.tensor([mine], dtype=torch.float64, device="cuda")
+                    allr = [torch.empty_like(t) for _ in range(world)]
+                    dist.all_gather(allr, t)
+                    callback = round(max(float(x) for x in allr), 3)
                 bd = breakdown(fn)
                 rec = {"tool": "bench_air_sharded", "case": name, "variant": vname, "gpus": world, "log_n": log_n, "width": width,
                        "opts": {k: int(v) for k, v in OPTS.items()}, "input": inp, "ms_per_proof": ms, "rank_steps_ms": per,
-                       "first_call_s": round(first_s, 3), "byte_identical_to_one_gpu": identical, "breakdown": bd,
+                       "first_call_s": round(first_s, 3), "byte_identical_to_one_gpu": identical, "callback_ms": callback, "breakdown": bd,
                        "stats": dict(stats) if world > 1 else None, "columns": [wf.shard_columns(width, world, q) for q in range(world)] if world > 1 else None,
                        "jit": ctx.jit_stats(), "card_before": before, "card_after": after,
                        "l2": "256 MiB memset before every timed step", "steps": a.steps, "warmup": a.warmup}

@@ -29,6 +29,7 @@ vp = C.c_void_p
 FRI_COMMIT_FN = C.CFUNCTYPE(None, C.c_void_p, u8p)
 FRI_DRAW_FN = C.CFUNCTYPE(None, C.c_void_p, u64p)
 AUX_BUILDER = C.CFUNCTYPE(C.c_int, C.c_void_p, u64p, u64p)
+AUX_SHARD_BUILDER = C.CFUNCTYPE(C.c_int, C.c_void_p, u64p, C.c_uint32, C.c_uint32, u64p)
 
 _lib = None
 
@@ -113,6 +114,8 @@ _SIGS = [
     ("wf_host_shard_columns", C.c_int, [C.c_uint32, C.c_int, C.c_int, C.POINTER(C.c_uint32), C.POINTER(C.c_uint32)]),
     ("wf_prove_air_sharded", C.c_int, [vp, vp, u64p, C.c_size_t, C.POINTER(u64p), vp, C.c_int, C.c_uint32, C.POINTER(C.c_uint32), u8p,
                                        C.POINTER(C.c_size_t), C.POINTER(C.c_double)]),
+    ("wf_prove_air_aux_sharded", C.c_int, [vp, vp, u64p, C.c_size_t, C.POINTER(u64p), vp, C.c_int, C.c_uint32, C.POINTER(C.c_uint32),
+                                           AUX_SHARD_BUILDER, AUX_BUILDER, vp, u8p, C.POINTER(C.c_size_t), C.POINTER(C.c_double)]),
 ]
 
 
@@ -589,6 +592,54 @@ def shard_columns(width, world, rank):
     if lib().wf_host_shard_columns(width, world, rank, C.byref(first), C.byref(count)) != WF_OK:
         raise WfError(f"wf_host_shard_columns: bad arguments (width {width}, world {world}, rank {rank})")
     return first.value, count.value
+
+
+def aux_shape(desc):
+    """(aux width, number of random elements, number of aux assertion values) of a flat AIR description (wf_prove_air_aux);
+    (0, 0, 0) without an aux segment or when the description is malformed (the library then refuses it)."""
+    d = [int(v) for v in np.asarray(desc, dtype=np.uint64).reshape(-1)]
+    p = 0
+
+    def rd(k=1):
+        nonlocal p
+        if p + k > len(d):
+            raise IndexError
+        p += k
+        return d[p - k]
+
+    def degrees():
+        for _ in range(rd()):
+            rd()
+            rd(rd())   # base, ncyc, cycles
+
+    try:
+        rd()                                     # width
+        degrees()
+        for _ in range(rd()):                    # periodic columns
+            rd(rd())
+        rd(rd())                                 # constants
+        rd()                                     # registers
+        rd(4 * rd())                             # program
+        for _ in range(rd()):                    # assertions: column, first_step, stride, nvals, values
+            rd(3)
+            rd(rd())
+        rd(rd())                                 # public inputs
+        rd()                                     # exemptions
+        if p == len(d):
+            return 0, 0, 0
+        aw, nr = rd(), rd()
+        degrees()
+        rd()
+        rd(4 * rd())
+        nv = 0
+        for _ in range(rd()):                    # aux assertions: values in E, three words each
+            rd(3)
+            k = rd()
+            rd(3 * k)
+            nv += k
+        return aw, nr, nv
+    except IndexError:
+        return 0, 0, 0
 
 
 def host_hash_elements(hash_id, elems):

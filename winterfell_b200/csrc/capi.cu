@@ -523,25 +523,32 @@ int wf_mat_from_device_columns(wf_ctx* ctx, const uint64_t* d_cols, uint32_t nco
     return WF_OK;
 }
 
-int wf_mat_from_host_columns(wf_ctx* ctx, const uint64_t* const* cols, uint32_t ncols, size_t nrows, int ext_degree,
-                             int mont, wf_mat** out) {
-    if (!ctx || !cols || !out || ncols == 0 || nrows == 0 || ext_degree < 1 || ext_degree > 3)
-        return wf_fail(ctx, WF_ERR_INVALID, "bad arguments");
-    // stage: host column j (nrows * d words, elements interleaved) -> device [ncols][nrows*d]
-    size_t col_words = nrows * ext_degree;
+// `nbase` base columns from host columns of d-component elements: base column q = component (q0 + q) % d of host column
+// (q0 + q) / d, so the block may start and end inside an element
+static int mat_from_host_elements(wf_ctx* ctx, const uint64_t* const* cols, uint32_t nbase, size_t nrows, int d, u32 q0, int mont,
+                                  wf_mat** out) {
+    // stage: host column j (nrows * d words, elements interleaved) -> device [ne][nrows*d]
+    const size_t col_words = nrows * d;
+    const u32 ne = (q0 + nbase - 1) / d + 1;
     void* stage;
-    CKI(wf_dev_alloc(ctx, (size_t)ncols * col_words * 8, &stage));
-    for (uint32_t j = 0; j < ncols; j++)
+    CKI(wf_dev_alloc(ctx, (size_t)ne * col_words * 8, &stage));
+    for (uint32_t j = 0; j < ne; j++)
         CK(cudaMemcpyAsync((u64*)stage + (size_t)j * col_words, cols[j], col_words * 8, cudaMemcpyHostToDevice, ctx->st));
     wf_mat* m;
-    int r = wf_mat_alloc(ctx, nrows, ncols * ext_degree, &m);
+    int r = wf_mat_alloc(ctx, nrows, nbase, &m);
     if (r != WF_OK) { wf_dev_free(ctx, stage); return r; }
-    // base column q = component (q % d) of column (q / d): element (row, q) at stage[(q/d)*col_words + row*d + q%d]
-    CK(layout_cols_to_seg((u64*)stage, nrows, ext_degree, mont, m->m, ctx->st));
+    // element (row, q) at stage[((q0+q)/d)*col_words + row*d + (q0+q)%d]
+    CK(layout_cols_to_seg((u64*)stage, nrows, d, mont, m->m, ctx->st, (int)q0));
     ctx->launches++;
     wf_dev_free(ctx, stage);
     *out = m;
     return WF_OK;
+}
+int wf_mat_from_host_columns(wf_ctx* ctx, const uint64_t* const* cols, uint32_t ncols, size_t nrows, int ext_degree,
+                             int mont, wf_mat** out) {
+    if (!ctx || !cols || !out || ncols == 0 || nrows == 0 || ext_degree < 1 || ext_degree > 3)
+        return wf_fail(ctx, WF_ERR_INVALID, "bad arguments");
+    return mat_from_host_elements(ctx, cols, ncols * ext_degree, nrows, ext_degree, 0, mont, out);
 }
 // Non-owning handle over caller-allocated device memory already in the segment layout of a rows x cols
 // matrix (segment width as for any matrix of `cols` columns: 8 for cols >= 8). wf_mat_free releases the
@@ -683,17 +690,22 @@ int wf_mat_lde_cosets(wf_ctx* ctx, const wf_mat* polys, uint32_t log_blowup, uin
 // compute stream. Columns are independent, so the result equals from_host_columns -> interpolate -> lde.
 int wf_trace_lde_from_host(wf_ctx* ctx, const uint64_t* const* cols, uint32_t ncols, size_t nrows, int mont, uint32_t log_blowup,
                            wf_mat** polys_out, wf_mat** lde_out) {
-    return wf_trace_lde_cosetwise(ctx, cols, nullptr, ncols, nrows, mont, log_blowup, polys_out, lde_out, false, nullptr, nullptr);
+    return wf_trace_lde_cosetwise(ctx, cols, nullptr, ncols, nrows, mont, log_blowup, polys_out, lde_out, false, nullptr, nullptr, 1, 0);
 }
 // The same pipeline with two knobs for the sharded prover (prover.cu): coset_major = the LDE is written coset-major
 // (row k * n + j = P(7 w_N^k w_n^j); *lde_out must then be preallocated, with the natural segment width of `ncols` columns or
 // a wider one: a rank of a sharded proof writes its columns at the segment width of the whole trace) and after_coset(k)
 // is called once coset k of ALL columns has been enqueued on the ctx stream — the caller starts that coset's exchange there.
 // d_cols != NULL: the columns are already on the device (column-major), no upload stage.
+// d > 1 (host columns only): cols are columns of d-component elements ([nrows][d] words each, as wf_mat_from_host_columns) and
+// the ncols BASE columns transformed are components q0, q0 + 1, ... of them: base column i = component (q0 + i) % d of host
+// column (q0 + i) / d (a rank's block of an auxiliary segment, which may start and end inside an element).
 int wf_trace_lde_cosetwise(wf_ctx* ctx, const uint64_t* const* cols, const uint64_t* d_cols, uint32_t ncols, size_t nrows, int mont,
                            uint32_t log_blowup, wf_mat** polys_out, wf_mat** lde_out, bool coset_major,
-                           const std::function<int(u32)>* after_coset, const LdeScatter* scatter) {
-    if (!ctx || (!cols && !d_cols) || !polys_out || (!lde_out && !scatter) || ncols == 0) return wf_fail(ctx, WF_ERR_INVALID, "bad arguments");
+                           const std::function<int(u32)>* after_coset, const LdeScatter* scatter, int d, uint32_t q0) {
+    if (!ctx || (!cols && !d_cols) || !polys_out || (!lde_out && !scatter) || ncols == 0 || d < 1 || d > 3 || q0 >= (u32)d ||
+        (d_cols && d != 1))
+        return wf_fail(ctx, WF_ERR_INVALID, "bad arguments");
     u32 log_n;
     if (log2_exact(nrows, &log_n) || log_n < 1) return wf_fail(ctx, WF_ERR_INVALID, "rows must be a power of two >= 2");
     if (log_blowup > 7 || log_n + log_blowup > 32) return wf_fail(ctx, WF_ERR_INVALID, "bad blowup");
@@ -730,7 +742,7 @@ int wf_trace_lde_cosetwise(wf_ctx* ctx, const uint64_t* const* cols, const uint6
     if (d_cols || Wc == 0 || log_n < 12) {  // resident columns, or too narrow / too small to be worth a pipeline
         wf_mat* tr;
         if (d_cols) CKI(wf_mat_from_device_columns(ctx, d_cols, ncols, nrows, &tr));
-        else CKI(wf_mat_from_host_columns(ctx, cols, ncols, nrows, 1, mont, &tr));
+        else CKI(mat_from_host_elements(ctx, cols, ncols, nrows, d, q0, mont, &tr));
         int r = wf_mat_interpolate(ctx, tr, polys_out);
         wf_mat_free(ctx, tr);
         if (r != WF_OK) return r;
@@ -762,7 +774,9 @@ int wf_trace_lde_cosetwise(wf_ctx* ctx, const uint64_t* const* cols, const uint6
         if (coset_major || scatter) lde = lde_out ? *lde_out : nullptr;
         else CKI(wf_mat_alloc(ctx, nrows << log_blowup, ncols, &lde));
         CKI(wf_mat_alloc_w(ctx, nrows, Wc, Wc, &tr));                       // one chunk of trace values (reused)
-        for (int i = 0; i < 2; i++) CKI(wf_dev_alloc(ctx, (size_t)Wc * nrows * 8, &stage[i]));
+        // a chunk of Wc base columns touches at most ne_max host columns of d components: each is uploaded whole
+        const size_t ne_max = (size_t)(Wc + d - 2) / d + 1;
+        for (int i = 0; i < 2; i++) CKI(wf_dev_alloc(ctx, ne_max * d * nrows * 8, &stage[i]));
         CKI(wf_dev_alloc(ctx, (size_t)Wc * nrows * 8, &tmp));               // two-pass scratch
         if (lde && lde->m.W > (int)ncols) CK(cudaMemsetAsync(lde->m.base, 0, lde->m.words() * 8, ctx->st));  // padding columns
         // the copy stream must not write pool buffers before their previous users on the compute stream are done
@@ -772,13 +786,15 @@ int wf_trace_lde_cosetwise(wf_ctx* ctx, const uint64_t* const* cols, const uint6
             const u32 c0 = k * Wc, cw = std::min<u32>(Wc, ncols - c0);
             const int sb = k & 1;
             if (k >= 2) CK(cudaStreamWaitEvent(ctx->copy_st, ctx->ev_used[sb], 0));
-            for (u32 j = 0; j < cw; j++)
-                CK(cudaMemcpyAsync((u64*)stage[sb] + (size_t)j * nrows, cols[c0 + j], nrows * 8, cudaMemcpyHostToDevice, ctx->copy_st));
+            const u32 e0 = (q0 + c0) / d, e1 = (q0 + c0 + cw - 1) / d;   // host columns holding base columns [c0, c0 + cw)
+            for (u32 e = e0; e <= e1; e++)
+                CK(cudaMemcpyAsync((u64*)stage[sb] + (size_t)(e - e0) * d * nrows, cols[e], (size_t)d * nrows * 8, cudaMemcpyHostToDevice,
+                                   ctx->copy_st));
             CK(cudaEventRecord(ctx->ev_up[sb], ctx->copy_st));
             CK(cudaStreamWaitEvent(ctx->st, ctx->ev_up[sb], 0));
             SegMatrix trv = tr->m;
             trv.cols = cw;
-            CK(layout_cols_to_seg((const u64*)stage[sb], nrows, 1, mont, trv, ctx->st));
+            CK(layout_cols_to_seg((const u64*)stage[sb], nrows, d, mont, trv, ctx->st, (int)((q0 + c0) % d)));
             CK(cudaEventRecord(ctx->ev_used[sb], ctx->st));
             ctx->launches++;
             SegMatrix pv = polys->m;                                          // segment k of the W = Wc polys matrix

@@ -143,7 +143,7 @@ struct LdeScatter {
 };
 extern "C" int wf_trace_lde_cosetwise(wf_ctx* ctx, const uint64_t* const* cols, const uint64_t* d_cols, uint32_t ncols, size_t nrows, int mont,
                            uint32_t log_blowup, wf_mat** polys_out, wf_mat** lde_out, bool coset_major,
-                           const std::function<int(u32)>* after_coset, const LdeScatter* scatter);
+                           const std::function<int(u32)>* after_coset, const LdeScatter* scatter, int d, uint32_t q0);
 extern "C" int wf_mat_lde_cosets(wf_ctx* ctx, const wf_mat* polys, uint32_t log_blowup, uint32_t k0, uint32_t k1, wf_mat* lde);  // internal (not in the public header)
 struct PublicCoin;
 struct Digest;

@@ -1,7 +1,7 @@
 // layout.cu — see layout.cuh.
 #include "layout.cuh"
 
-__global__ void __launch_bounds__(256) cols_to_seg_kernel(const u64* __restrict__ src, size_t nrows, int d, int mont,
+__global__ void __launch_bounds__(256) cols_to_seg_kernel(const u64* __restrict__ src, size_t nrows, int d, int q0, int mont,
                                                           SegMatrix dst) {
     // thread = (row, segment); reads W columns at `row` (coalesced per column across the warp),
     // writes one W*8-byte segment row. All W loads are issued before the first use: the kernel is a pure
@@ -13,8 +13,8 @@ __global__ void __launch_bounds__(256) cols_to_seg_kernel(const u64* __restrict_
     u64 v[8];
 #pragma unroll
     for (int q = 0; q < 8; q++) {
-        u32 col = g * dst.W + q;
-        v[q] = (q < dst.W && col < dst.cols) ? __ldg(src + (size_t)(col / d) * nrows * d + row * d + (col % d)) : 0;
+        u32 col = g * dst.W + q, sc = col + (u32)q0;   // base column `col` = component sc % d of source column sc / d
+        v[q] = (q < dst.W && col < dst.cols) ? __ldg(src + (size_t)(sc / d) * nrows * d + row * d + (sc % d)) : 0;
     }
     if (mont) {
 #pragma unroll
@@ -108,8 +108,8 @@ __global__ void __launch_bounds__(256) select_cols_kernel(SegMatrix src, u32 fir
 
 static dim3 row_grid(size_t rows, u32 nseg) { return dim3((unsigned)((rows + 255) / 256), nseg); }
 
-cudaError_t layout_cols_to_seg(const u64* src, size_t nrows, int d, int mont, const SegMatrix& dst, cudaStream_t st) {
-    cols_to_seg_kernel<<<row_grid(nrows, dst.nseg()), 256, 0, st>>>(src, nrows, d, mont, dst);
+cudaError_t layout_cols_to_seg(const u64* src, size_t nrows, int d, int mont, const SegMatrix& dst, cudaStream_t st, int q0) {
+    cols_to_seg_kernel<<<row_grid(nrows, dst.nseg()), 256, 0, st>>>(src, nrows, d, q0, mont, dst);
     return cudaGetLastError();
 }
 cudaError_t layout_rows_to_seg(const u64* src, const SegMatrix& dst, cudaStream_t st) {

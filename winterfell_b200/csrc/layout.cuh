@@ -6,8 +6,9 @@
 #include "commit.cuh"
 
 // src: columns of `d`-degree elements, column j at src[j * nrows * d ...], element (row, comp) at
-// row * d + comp. Base column q = component q % d of column q / d. mont: words are Montgomery form.
-cudaError_t layout_cols_to_seg(const u64* src, size_t nrows, int d, int mont, const SegMatrix& dst, cudaStream_t st);
+// row * d + comp. Base column q = component (q0 + q) % d of column (q0 + q) / d: q0 < d skips the first components of
+// column 0 (a block of base columns that starts inside an element). mont: words are Montgomery form.
+cudaError_t layout_cols_to_seg(const u64* src, size_t nrows, int d, int mont, const SegMatrix& dst, cudaStream_t st, int q0 = 0);
 // src: row-major [rows][cols]
 cudaError_t layout_rows_to_seg(const u64* src, const SegMatrix& dst, cudaStream_t st);
 // dst: column-major [cols][rows] (row_major = 0) or row-major [rows][cols] (row_major = 1)

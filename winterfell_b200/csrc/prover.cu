@@ -1577,59 +1577,42 @@ static int sharded_shape_check(wf_ctx* ctx, const AirHost& air, u32 log_n, const
     return WF_OK;
 }
 
-// One proof of a single-segment AIR sharded over the ranks of `cm` (wf_prove_fib_sharded, wf_prove_air_sharded). The
-// arguments have been checked on every rank alike; this rank passes the columns shard_columns assigns it (none is possible).
-template <int D>
-int prove_sharded(wf_ctx* ctx, const wf_comm* cm, const AirHost& air, const uint64_t* const* local_cols, const uint64_t* d_local, int mont,
-                  u32 log_n, const Options& o, std::vector<u8>& proof_out, double* stats) {
-    ShardCtx sc{ctx, cm, cm->world, cm->rank, 0};
-    const int G = sc.G, r = sc.r;
-    CKI(sharded_shape_check(ctx, air, log_n, o, G, r));
-    while ((1 << sc.logG) < G) sc.logG++;
-    const int h = o.hash_id;
-    const size_t n = (size_t)1 << log_n;
-    u32 log_b = 0;
-    while ((1u << log_b) < o.blowup) log_b++;
-    const size_t N = n << log_b, b = o.blowup;
-    const u32 c = air.w;
-    const u32 kc = air.num_comp_cols(n), log_ceb = air.log_ce_blowup();
-    const size_t rows_per = N / (size_t)G, ce = n << log_ceb, ce_per = ce / (size_t)G;
-    // Column ownership, in segments of the WHOLE trace's width Wg: the row shard, the staging buffer and every rank's local LDE
-    // use that width, so local segment g of rank q is global segment sg0[q] + g and blocks move as whole segment rows
-    const int Wg = seg_width_for(c);
-    const u32 nsg = (c + Wg - 1) / Wg;
-    std::vector<u32> col0(G), ncol(G), sg0(G), nsl(G);
-    for (int q = 0; q < G; q++) {
-        shard_columns(c, G, q, &col0[q], &ncol[q]);
-        sg0[q] = col0[q] / Wg;
-        nsl[q] = (ncol[q] + Wg - 1) / Wg;
+// Column ownership of one trace segment (shard_columns), in segments of the WHOLE segment's width Wg: the row shard, the staging
+// buffer and every rank's local LDE use that width, so local segment g of rank q is global segment sg0[q] + g and blocks move
+// as whole segment rows
+struct ShardSplit {
+    u32 c, nsg;
+    int Wg;
+    std::vector<u32> col0, ncol, sg0, nsl;
+    ShardSplit(u32 cols, int G) : c(cols), Wg(seg_width_for(cols)), col0(G), ncol(G), sg0(G), nsl(G) {
+        nsg = (c + Wg - 1) / Wg;
+        for (int q = 0; q < G; q++) {
+            shard_columns(c, G, q, &col0[q], &ncol[q]);
+            sg0[q] = col0[q] / Wg;
+            nsl[q] = (ncol[q] + Wg - 1) / Wg;
+        }
     }
-    const u32 cl = ncol[r];
-    const u32 n_tr = (u32)air.degrees.size(), n_as = (u32)air.asserts.size();
-    Channel<D> ch(h, channel_seed(air, n, o));  // every rank replays the whole transcript
+};
 
-    wf_mat *trace = nullptr, *polys = nullptr, *lde = nullptr, *shard = nullptr, *comp_l = nullptr, *comp = nullptr, *cpolys = nullptr,
-           *clde = nullptr, *deep = nullptr, *fri_in = nullptr, *tstage = nullptr;
-    ShardTree ttree, ctree;
-    wf_fri* fri = nullptr;
-    ProofScope scope(ctx);   // holds the ADDRESSES of these pointers: every owned pointer lives as long as the scope
-    scope.own({&trace, &polys, &lde, &shard, &comp_l, &comp, &cpolys, &clde, &deep, &fri_in, &tstage});
-    scope.own({&ttree.local, &ctree.local});
-    scope.fri = &fri;
-    struct SLayer { u64* vals; size_t m_l, m_g; ShardTree tree; };
-    std::vector<SLayer> slayers;   // FRI layers folded on row shards
-    std::vector<void*> owned;      // device buffers of the sharded FRI phase
-    struct Cleanup {
-        wf_ctx* ctx; std::vector<SLayer>& sl; std::vector<void*>& ow;
-        ~Cleanup() { for (auto& l : sl) wf_tree_free(ctx, l.tree.local); for (void* p : ow) wf_dev_free(ctx, p); }
-    } cleanup{ctx, slayers, owned};
-
-    // ---- 1. interpolate the local columns, then extend them coset by coset (no communication: columns are independent).
+// One trace segment from this rank's columns to its row shard: interpolate the local base columns, extend them coset by coset
+// (no communication: columns are independent) and move every rank's rows to it. *shard_out = LDE rows [r N/G, (r+1) N/G) of
+// every column of the segment followed by `blowup` halo rows (the first rows of rank r + 1); *polys_out = the local columns'
+// polynomials (none when the rank owns no column). Columns: resident d_local, or host columns of d-component elements starting
+// at component q0 (wf_trace_lde_cosetwise). *path = the transport that ran: 2 fused scatter, 1 peer copies, 0 exchange.
+static int segment_to_row_shard(ShardCtx& sc, const ShardSplit& sp, const uint64_t* const* cols, const uint64_t* d_local, int d, u32 q0,
+                                int mont, u32 log_n, u32 log_b, wf_mat** polys_out, wf_mat** shard_out, int* path, const char* mark_lde) {
+    wf_ctx* ctx = sc.ctx;
+    const int G = sc.G, r = sc.r, Wg = sp.Wg;
+    const u32 c = sp.c, nsg = sp.nsg, cl = sp.ncol[r];
+    const std::vector<u32>&sg0 = sp.sg0, &nsl = sp.nsl;
+    const size_t n = (size_t)1 << log_n, b = (size_t)1 << log_b, N = n << log_b, rows_per = N / (size_t)G;
     //         Coset k is written coset-major, so that the rows of rank q's range (n / G points of the coset) are one contiguous
-    //         block per segment: its exchange runs on the communicator's stream while coset k + 1 is being extended ----
-    wf_mark(ctx, "start");
+    //         block per segment: its exchange runs on the communicator's stream while coset k + 1 is being extended
     const size_t nj = n / (size_t)G;   // points of one coset inside one rank's row range
     const size_t blk = nj * (size_t)Wg * 8;   // bytes of one (segment, coset, row range) block
+    wf_mat *&polys = *polys_out, *&shard = *shard_out, *lde = nullptr, *stage = nullptr;
+    ProofScope tmp(ctx);   // this segment's local LDE and staging buffer
+    tmp.own({&lde, &stage});
     CKI(wf_mat_alloc(ctx, rows_per + b, c, &shard));   // segment width Wg
     shard->m.rows = rows_per;  // seg_stride stays (rows_per + b) * Wg: rows [rows_per, rows_per + b) are the halo
     const size_t sstride = shard->m.seg_stride;
@@ -1652,17 +1635,17 @@ int prove_sharded(wf_ctx* ctx, const wf_comm* cm, const AirHost& air, const uint
         LdeScatter sct;
         for (int q = 0; q < 8; q++) sct.peer[q] = q < G ? (u64*)peer_shard[q] : nullptr;
         sct.seg_stride = sstride; sct.seg0 = sg0[r]; sct.log_nj = log_nj; sct.world = (u32)G;
-        CKI(wf_trace_lde_cosetwise(ctx, local_cols, d_local, cl, n, mont, log_b, &polys, nullptr, false, nullptr, &sct));
-        wf_mark(ctx, "trace_lde");
+        CKI(wf_trace_lde_cosetwise(ctx, cols, d_local, cl, n, mont, log_b, &polys, nullptr, false, nullptr, &sct, d, q0));
+        wf_mark(ctx, mark_lde);
         CK(cudaStreamSynchronize(ctx->st));   // my stores have landed; everybody's have when every rank says so
         CKI(sc.host_barrier());
         sc.ncoll += 1;
         sc.bytes_overlapped += (double)(G - 1) * nsl[r] * (double)rows_per * Wg * 8;
-        push = true;
-    } else {
-    wf_mat*& stage = tstage;           // what arrives: [global segment][coset][nj][Wg]
+        *path = 2;
+        return WF_OK;
+    }
     if (cl) CKI(wf_mat_alloc_w(ctx, N, cl, Wg, &lde));   // mine, coset-major: [local segment][coset][n][Wg]
-    CKI(wf_mat_alloc_w(ctx, rows_per, c, Wg, &stage));
+    CKI(wf_mat_alloc_w(ctx, rows_per, c, Wg, &stage));   // what arrives: [global segment][coset][nj][Wg]
     // Preferred transport: every rank maps the others' `stage` buffers (CUDA IPC) and PUSHES its blocks there with peer copies
     // on side streams — copy engines over NVLink, no SM taken from the NTT kernels they overlap (NCCL send/recv kernels on a
     // side stream were measured: they slow the LDE down by as much as they hide). Fallback: the communicator's exchange.
@@ -1692,25 +1675,25 @@ int prove_sharded(wf_ctx* ctx, const wf_comm* cm, const AirHost& air, const uint
             return WF_OK;
         }
         // pairwise order: sender r -> q lists my segments ascending; receiver r <- q lists q's segments ascending
-        std::vector<int> sp, rp;
+        std::vector<int> spk, rp;
         std::vector<const void*> sv;
         std::vector<void*> rv;
         for (u32 sg = 0; sg < nsl[r]; sg++)
             for (int q = 0; q < G; q++) {
                 if (q == r) CK(cudaMemcpyAsync(stage_block(stage->m.base, sg0[r] + sg, k), my_block(sg, k, r), blk, cudaMemcpyDeviceToDevice, ctx->st));
-                else { sp.push_back(q); sv.push_back(my_block(sg, k, q)); }
+                else { spk.push_back(q); sv.push_back(my_block(sg, k, q)); }
             }
         for (int q = 0; q < G; q++)
             for (u32 sg = 0; q != r && sg < nsl[q]; sg++) { rp.push_back(q); rv.push_back(stage_block(stage->m.base, sg0[q] + sg, k)); }
         CKI(sc.fork());
-        return sc.exchange(sp, sv, rp, rv, blk);
+        return sc.exchange(spk, sv, rp, rv, blk);
     };
     // (upload ->) layout -> interpolate -> extend, pipelined per column chunk for host columns; the cosets of the last chunk
     // are extended one by one and after_coset(k) ships coset k while coset k + 1 is computed. A rank without columns only
     // takes part in the exchanges.
-    if (cl) CKI(wf_trace_lde_cosetwise(ctx, local_cols, d_local, cl, n, mont, log_b, &polys, &lde, true, &after_coset, nullptr));
+    if (cl) CKI(wf_trace_lde_cosetwise(ctx, cols, d_local, cl, n, mont, log_b, &polys, &lde, true, &after_coset, nullptr, d, q0));
     else for (u32 k = 0; k < (u32)b; k++) CKI(after_coset(k));
-    wf_mark(ctx, "trace_lde");
+    wf_mark(ctx, mark_lde);
     if (push) {
         // my pushes have landed when my side streams drain; everybody's have when every rank says so
         for (int i = 0; i < 4; i++) CK(cudaStreamSynchronize(ctx->push_st[i]));
@@ -1726,8 +1709,8 @@ int prove_sharded(wf_ctx* ctx, const wf_comm* cm, const AirHost& air, const uint
         ctx->launches++;
         CK(cudaGetLastError());
     }
-    scope.drop(lde);
-    scope.drop(stage);
+    tmp.drop(lde);
+    tmp.drop(stage);
     {   // halo: the first `blowup` rows of every segment of rank (r + 1) mod G
         void *pk, *pk2;
         const size_t hb = b * Wg * 8;
@@ -1739,7 +1722,64 @@ int prove_sharded(wf_ctx* ctx, const wf_comm* cm, const AirHost& air, const uint
         wf_dev_free(ctx, pk);
         wf_dev_free(ctx, pk2);
     }
-    }
+    *path = push ? 1 : 0;
+    return WF_OK;
+}
+
+// FNV-1a, for the agreement steps of a sharded proof: what must be equal on every rank is hashed and the hashes all-gathered
+struct Fnv {
+    u64 h = 0xcbf29ce484222325ULL;
+    void mix(u64 v) { for (int i = 0; i < 8; i++) { h ^= (v >> (8 * i)) & 0xff; h *= 0x100000001b3ULL; } }
+};
+
+// One proof sharded over the ranks of `cm` (wf_prove_fib_sharded, wf_prove_air_sharded, wf_prove_air_aux_sharded). The
+// arguments have been checked on every rank alike; this rank passes the main columns shard_columns assigns it (none is
+// possible) and, for a two-segment AIR, builds the aux columns it owns with aux_builder.
+template <int D>
+int prove_sharded(wf_ctx* ctx, const wf_comm* cm, const AirHost& air_in, const uint64_t* const* local_cols, const uint64_t* d_local, int mont,
+                  u32 log_n, const Options& o, std::vector<u8>& proof_out, double* stats, wf_aux_shard_builder_fn aux_builder = nullptr,
+                  wf_aux_assertions_fn aux_assertions = nullptr, void* aux_user = nullptr) {
+    AirHost air_dyn;                       // copy whose aux assertion values are rewritten from the random elements (as prove_air)
+    if (aux_assertions) air_dyn = air_in;
+    const AirHost& air = aux_assertions ? air_dyn : air_in;
+    ShardCtx sc{ctx, cm, cm->world, cm->rank, 0};
+    const int G = sc.G, r = sc.r;
+    CKI(sharded_shape_check(ctx, air, log_n, o, G, r));
+    while ((1 << sc.logG) < G) sc.logG++;
+    const int h = o.hash_id;
+    const size_t n = (size_t)1 << log_n;
+    u32 log_b = 0;
+    while ((1u << log_b) < o.blowup) log_b++;
+    const size_t N = n << log_b;
+    const u32 c = air.w, aw = air.aw;
+    const u32 kc = air.num_comp_cols(n), log_ceb = air.log_ce_blowup();
+    const size_t rows_per = N / (size_t)G, ce = n << log_ceb, ce_per = ce / (size_t)G;
+    const ShardSplit tsp(c, G), asp(aw * D, G);   // main columns; aux BASE columns (component q of E column j = j D + q)
+    const std::vector<u32>&col0 = tsp.col0, &ncol = tsp.ncol;
+    const u32 cl = ncol[r], acl = aw ? asp.ncol[r] : 0;
+    const u32 n_tr = (u32)(air.degrees.size() + air.aux_degrees.size()), n_as = (u32)(air.asserts.size() + air.aux_asserts.size());
+    Channel<D> ch(h, channel_seed(air, n, o));  // every rank replays the whole transcript
+
+    wf_mat *polys = nullptr, *shard = nullptr, *apolys = nullptr, *ashard = nullptr, *comp_l = nullptr, *comp = nullptr, *cpolys = nullptr,
+           *clde = nullptr, *deep = nullptr, *fri_in = nullptr;
+    ShardTree ttree, atree, ctree;
+    wf_fri* fri = nullptr;
+    ProofScope scope(ctx);   // holds the ADDRESSES of these pointers: every owned pointer lives as long as the scope
+    scope.own({&polys, &shard, &apolys, &ashard, &comp_l, &comp, &cpolys, &clde, &deep, &fri_in});
+    scope.own({&ttree.local, &atree.local, &ctree.local});
+    scope.fri = &fri;
+    struct SLayer { u64* vals; size_t m_l, m_g; ShardTree tree; };
+    std::vector<SLayer> slayers;   // FRI layers folded on row shards
+    std::vector<void*> owned;      // device buffers of the sharded FRI phase
+    struct Cleanup {
+        wf_ctx* ctx; std::vector<SLayer>& sl; std::vector<void*>& ow;
+        ~Cleanup() { for (auto& l : sl) wf_tree_free(ctx, l.tree.local); for (void* p : ow) wf_dev_free(ctx, p); }
+    } cleanup{ctx, slayers, owned};
+
+    // ---- 1-2. main trace: local columns -> LDE -> row shard with halo ----
+    wf_mark(ctx, "start");
+    int tpath = 0, apath = 0;
+    CKI(segment_to_row_shard(sc, tsp, local_cols, d_local, 1, 0, mont, log_n, log_b, &polys, &shard, &tpath, "trace_lde"));
     wf_mark(ctx, "trace_exchange");
     // ---- 3. leaves + subtree over my rows, all-gather of the subtree roots ----
     Digest root;
@@ -1748,15 +1788,76 @@ int prove_sharded(wf_ctx* ctx, const wf_comm* cm, const AirHost& air, const uint
     CKI(shard_tree_finish(sc, h, ttree, &root));
     wf_mark(ctx, "trace_commit");
     ch.commit(root.b);
-    // ---- 4. constraint evaluation over my CE rows ----
+    // ---- 3b. auxiliary segment (prove_air 1b): every rank draws the random elements and builds the E columns that cover its
+    //          aux base columns (an E column split between two ranks is built by both), the ranks agree on the callbacks'
+    //          outcome, then the segment goes the main trace's way: LDE, row shard with halo, subtree, commitment ----
+    std::vector<u64> rnd_flat;  // [nr][D], canonical
+    double cb_ms = 0;
+    if (aw) {
+        for (u32 i = 0; i < air.nr; i++) { GlExt<D> e = ch.draw(); for (int q = 0; q < D; q++) rnd_flat.push_back(e.v[q]); }
+        std::vector<u64> rnd_user = rnd_flat;
+        if (mont) for (u64& v : rnd_user) v = gl_mul(v, 0xFFFFFFFFULL);  // x * R, R = 2^64 mod p
+        const u32 af = asp.col0[r], e0 = af / D, ne = acl ? (af + acl + D - 1) / D - e0 : 0;
+        std::vector<u64> aux_host((size_t)ne * n * D);  // [ne][n][D]: E columns [e0, e0 + ne)
+        int st = WF_OK;
+        const auto t0 = std::chrono::steady_clock::now();
+        if (ne && aux_builder(aux_user, rnd_user.data(), e0, ne, aux_host.data()) != 0)
+            st = wf_fail(ctx, WF_ERR_INVALID, "aux trace builder failed (rank %d, columns [%u, %u))", r, e0, e0 + ne);
+        if (st == WF_OK && aux_assertions) {
+            size_t total = 0;
+            for (auto& a : air_dyn.aux_asserts) total += a.values.size() / 3;
+            std::vector<u64> vals(total * D);
+            size_t q = 0;
+            for (auto& a : air_dyn.aux_asserts)
+                for (size_t i = 0; i < a.values.size() / 3; i++, q++)
+                    for (int k = 0; k < D; k++) vals[q * D + k] = mont ? gl_mul(a.values[i * 3 + k], 0xFFFFFFFFULL) : a.values[i * 3 + k];
+            if (aux_assertions(aux_user, rnd_user.data(), vals.data()) != 0) st = wf_fail(ctx, WF_ERR_INVALID, "aux assertion callback failed");
+            q = 0;
+            for (auto& a : air_dyn.aux_asserts)
+                for (size_t i = 0; st == WF_OK && i < a.values.size() / 3; i++, q++)
+                    for (int k = 0; st == WF_OK && k < 3; k++) {
+                        u64 v = k < D ? vals[q * D + k] : 0;
+                        if (mont) v = gl_from_mont(v);
+                        else if (v >= GL_P) st = wf_fail(ctx, WF_ERR_INVALID, "aux assertion value is not a canonical field element");
+                        a.values[i * 3 + k] = v;
+                    }
+        }
+        cb_ms = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count();
+        wf_mark(ctx, "aux_build");
+        // agreement: every rank takes the same way out of here, even when only one rank's callback failed
+        Fnv vh;
+        for (auto& a : air.aux_asserts) for (u64 v : a.values) vh.mix(v);
+        struct Vote { int32_t status, pad; u64 hash; } v{st, 0, vh.h};
+        std::vector<Vote> all(G);
+        CKI(sc.gather_host(&v, all.data(), sizeof(Vote)));
+        for (int q = 0; q < G; q++) {   // the lowest failing rank's status, on every rank
+            if (all[q].status == WF_OK) continue;
+            if (q == r) return st;
+            return wf_fail(ctx, all[q].status, "rank %d's aux callbacks failed", q);
+        }
+        for (int q = 0; q < G; q++)
+            if (all[q].hash != vh.h) return wf_fail(ctx, WF_ERR_INVALID, "ranks %d and %d computed different aux assertion values", r, q);
+        std::vector<const u64*> ecols(ne);   // E column e0 + j -> base columns (e0 + j) D + q; mine start at component af % D
+        for (u32 j = 0; j < ne; j++) ecols[j] = &aux_host[(size_t)j * n * D];
+        CKI(segment_to_row_shard(sc, asp, ne ? ecols.data() : nullptr, nullptr, D, af % D, mont, log_n, log_b, &apolys, &ashard, &apath,
+                                 "aux_lde"));
+        wf_mark(ctx, "aux_exchange");
+        CKI(wf_commit_rows_partitioned(ctx, h, ashard, o.part_words(aw, D), &atree.local));
+        atree.n_global = N;
+        CKI(shard_tree_finish(sc, h, atree, &root));
+        wf_mark(ctx, "aux_commit");
+        ch.commit(root.b);
+    }
+    // ---- 4. constraint evaluation over my CE rows; coefficient order as prove_air's ----
     std::vector<GlExt<D>> cc = ch.draw_coeffs(o.batch_c, n_tr + n_as);
-    CKI(eval_constraints<D>(ctx, air, shard, nullptr, cc, {}, log_n, log_b, &comp_l, (size_t)r * ce_per, ce_per));
+    CKI(eval_constraints<D>(ctx, air, shard, ashard, cc, rnd_flat, log_n, log_b, &comp_l, (size_t)r * ce_per, ce_per));
     wf_mark(ctx, "constraint_eval");
     // ---- 5. composition polynomial: all-gather the CE evaluations (a few hundred MiB at most), interpolate + extend on
     //         every rank (the transform is over the row index), commit my row range ----
     CKI(wf_mat_alloc(ctx, ce, D, &comp));
     CKI(sc.all_gather_dev(comp_l->m.base, comp->m.base, ce_per * comp->m.W * 8));
     scope.drop(comp_l);
+    const size_t b = o.blowup;
     wf_mat cview;  // my rows of the composition LDE
     if (b % (size_t)G == 0) {
         // the composition polynomial has too few columns to shard by column: shard its LDE by COSET instead. Rank r extends
@@ -1823,22 +1924,33 @@ int prove_sharded(wf_ctx* ctx, const wf_comm* cm, const AirHost& air, const uint
     //         column count: the gather takes equal sizes); composition columns are replicated ----
     GlExt<D> z = ch.draw();
     GlExt<D> zg = ext_mul_base(z, gl_root_of_unity(log_n));
-    std::vector<std::vector<GlExt<D>>> ood;   // [0], [1]: composition columns at z, zg; [2], [3]: my trace columns
+    std::vector<std::vector<GlExt<D>>> ood;   // [0], [1]: composition columns at z, zg; then my trace columns, my aux base columns
     std::vector<const wf_mat*> om = {cpolys};
     if (cl) om.push_back(polys);
+    if (acl) om.push_back(apolys);
     CKI(ood_eval<D>(ctx, om, z, zg, ood));
-    std::vector<GlExt<D>> t_cur(c), t_nxt(c);
+    std::vector<GlExt<D>> t_cur(c), t_nxt(c), ab_cur((size_t)aw * D), ab_nxt((size_t)aw * D);   // ab_*: per aux base column
     {
-        const u32 cmax = *std::max_element(ncol.begin(), ncol.end());
-        std::vector<u64> mine((size_t)cmax * 2 * D, 0), all((size_t)G * cmax * 2 * D);
-        for (u32 j = 0; j < cl; j++)
-            for (int q = 0; q < D; q++) { mine[((size_t)j * 2) * D + q] = ood[2][j].v[q]; mine[((size_t)j * 2 + 1) * D + q] = ood[3][j].v[q]; }
+        const u32 cmax = *std::max_element(ncol.begin(), ncol.end()), amax = *std::max_element(asp.ncol.begin(), asp.ncol.end());
+        const u32 amx = aw ? amax : 0, per = cmax + amx;   // one rank's part: its main columns, then its aux base columns
+        std::vector<u64> mine((size_t)per * 2 * D, 0), all((size_t)G * per * 2 * D);
+        auto put = [&](u32 slot, const GlExt<D>& x0, const GlExt<D>& x1) {
+            for (int q = 0; q < D; q++) { mine[((size_t)slot * 2) * D + q] = x0.v[q]; mine[((size_t)slot * 2 + 1) * D + q] = x1.v[q]; }
+        };
+        for (u32 j = 0; j < cl; j++) put(j, ood[2][j], ood[3][j]);
+        const size_t ai = cl ? 4 : 2;
+        for (u32 j = 0; j < acl; j++) put(cmax + j, ood[ai][j], ood[ai + 1][j]);
         CKI(sc.gather_host(mine.data(), all.data(), mine.size() * 8));
-        for (int rq = 0; rq < G; rq++)
+        for (int rq = 0; rq < G; rq++) {
             for (u32 j = 0; j < ncol[rq]; j++) {
-                const u64* e = &all[((size_t)rq * cmax + j) * 2 * D];
+                const u64* e = &all[((size_t)rq * per + j) * 2 * D];
                 for (int q = 0; q < D; q++) { t_cur[col0[rq] + j].v[q] = e[q]; t_nxt[col0[rq] + j].v[q] = e[D + q]; }
             }
+            for (u32 j = 0; aw && j < asp.ncol[rq]; j++) {
+                const u64* e = &all[((size_t)rq * per + cmax + j) * 2 * D];
+                for (int q = 0; q < D; q++) { ab_cur[asp.col0[rq] + j].v[q] = e[q]; ab_nxt[asp.col0[rq] + j].v[q] = e[D + q]; }
+            }
+        }
     }
     auto combine = [&](const std::vector<GlExt<D>>& comp_evals) {  // H_j(z) from its base-component columns
         std::vector<GlExt<D>> rr(comp_evals.size() / D);
@@ -1854,6 +1966,12 @@ int prove_sharded(wf_ctx* ctx, const wf_comm* cm, const AirHost& air, const uint
         return rr;
     };
     std::vector<GlExt<D>> q_cur = combine(ood[0]), q_nxt = combine(ood[1]);
+    if (aw) {  // trace frame rows = main columns then aux columns; an E column's components may come from two ranks
+        auto a_cur = combine(ab_cur), a_nxt = combine(ab_nxt);
+        t_cur.insert(t_cur.end(), a_cur.begin(), a_cur.end());
+        t_nxt.insert(t_nxt.end(), a_nxt.begin(), a_nxt.end());
+    }
+    const u32 ct = c + aw;
     ByteVec ood_t, ood_q;
     ood_t.u8_(2); write_elems<D>(ood_t, t_cur); write_elems<D>(ood_t, t_nxt);
     ood_q.u8_(2); write_elems<D>(ood_q, q_cur); write_elems<D>(ood_q, q_nxt);
@@ -1865,11 +1983,11 @@ int prove_sharded(wf_ctx* ctx, const wf_comm* cm, const AirHost& air, const uint
     }
     wf_mark(ctx, "ood_frames");
     // ---- 7. DEEP composition over my LDE rows (evaluation form is row-local) ----
-    std::vector<GlExt<D>> dc = ch.draw_coeffs(o.batch_d, c + kc);
+    std::vector<GlExt<D>> dc = ch.draw_coeffs(o.batch_d, ct + kc);
     GlExt<D> Sz = ext_zero<D>(), Szg = ext_zero<D>();
-    for (u32 j = 0; j < c; j++) { Sz = ext_add(Sz, ext_mul(dc[j], t_cur[j])); Szg = ext_add(Szg, ext_mul(dc[j], t_nxt[j])); }
-    for (u32 j = 0; j < kc; j++) { Sz = ext_add(Sz, ext_mul(dc[c + j], q_cur[j])); Szg = ext_add(Szg, ext_mul(dc[c + j], q_nxt[j])); }
-    CKI(deep_compose<D>(ctx, shard, nullptr, &cview, kc, log_n + log_b, dc, z, zg, Sz, Szg, &deep, (size_t)r * rows_per, rows_per));
+    for (u32 j = 0; j < ct; j++) { Sz = ext_add(Sz, ext_mul(dc[j], t_cur[j])); Szg = ext_add(Szg, ext_mul(dc[j], t_nxt[j])); }
+    for (u32 j = 0; j < kc; j++) { Sz = ext_add(Sz, ext_mul(dc[ct + j], q_cur[j])); Szg = ext_add(Szg, ext_mul(dc[ct + j], q_nxt[j])); }
+    CKI(deep_compose<D>(ctx, shard, ashard, &cview, kc, log_n + log_b, dc, z, zg, Sz, Szg, &deep, (size_t)r * rows_per, rows_per));
     wf_mark(ctx, "deep_composition");
     // ---- 8. FRI: layers folded on shards while they are large. A layer of L points is held as contiguous position
     //         ranges; leaf i joins positions i, i + L/nf, ...: one exchange gives the owner of leaf range o (L/nf/G leaves)
@@ -1960,13 +2078,16 @@ int prove_sharded(wf_ctx* ctx, const wf_comm* cm, const AirHost& air, const uint
         for (size_t i = 0; i < p.size(); i++) if ((int)(p[i] / per) == r) l[i] = p[i] % per;
         return l;
     };
-    std::vector<std::pair<size_t, u64>> top_t, top_c;
+    std::vector<std::pair<size_t, u64>> top_t, top_a, top_c;
     size_t tr_rows = gb.add_rows(shard->m, owned_rows(pos, rows_per));
+    size_t ar_rows = 0, ar_dig = 0;
+    if (aw) ar_rows = gb.add_rows(ashard->m, owned_rows(pos, rows_per));
     size_t cr_rows = comp_sharded ? gb.add_rows(cview.m, owned_rows(pos, rows_per))
                                   : gb.add_rows(clde->m, r == 0 ? pos : std::vector<u64>(pos.size(), NONE));  // replicated: rank 0 contributes
     size_t tr_dig, cr_dig;
     CKI(gb.add_opening_sharded(ctx, ttree.local, N, G, r, pos, &tr_dig, &top_t));
     CKI(gb.add_opening_sharded(ctx, ctree.local, N, G, r, pos, &cr_dig, &top_c));
+    if (aw) CKI(gb.add_opening_sharded(ctx, atree.local, N, G, r, pos, &ar_dig, &top_a));
     struct SQ { size_t row_id, dig_id, nq; std::vector<std::pair<size_t, u64>> top; };
     std::vector<SQ> sq;
     std::vector<u64> fpos = pos;
@@ -2001,8 +2122,10 @@ int prove_sharded(wf_ctx* ctx, const wf_comm* cm, const AirHost& air, const uint
     };
     patch(tr_dig, top_t, ttree);
     patch(cr_dig, top_c, ctree);
+    if (aw) patch(ar_dig, top_a, atree);
     for (size_t i = 0; i < sq.size(); i++) patch(sq[i].dig_id, sq[i].top, slayers[i].tree);
     write_queries(gb, tr_rows, tr_dig, pos.size() * c, w);
+    if (aw) write_queries(gb, ar_rows, ar_dig, pos.size() * aw * D, w);
     write_queries(gb, cr_rows, cr_dig, pos.size() * kc * D, w);
     w.u16_((uint16_t)ood_t.v.size()); w.bytes(ood_t.v.data(), ood_t.v.size());
     w.u16_((uint16_t)ood_q.v.size()); w.bytes(ood_q.v.data(), ood_q.v.size());
@@ -2039,7 +2162,8 @@ int prove_sharded(wf_ctx* ctx, const wf_comm* cm, const AirHost& air, const uint
         for (int i = 4; i < 8; i++) stats[i] = 0;
         stats[4] = (double)slayers.size();
         stats[5] = sc.bytes_overlapped;
-        stats[6] = scat ? 2.0 : (push ? 1.0 : 0.0);
+        stats[6] = (double)tpath;   // the main trace's transport (the aux segment's: its own split decides)
+        stats[7] = cb_ms;
     }
     return WF_OK;
 }
@@ -2293,13 +2417,14 @@ extern "C" int wf_deep_compose(wf_ctx* ctx, uint32_t ext, const wf_mat* main_lde
 
 static int prove_sharded_dispatch(wf_ctx* ctx, const wf_comm* comm, const AirHost& air, const uint64_t* const* local_cols,
                                   const uint64_t* d_local, int mont, uint32_t log_n, const Options& o, uint8_t* proof, size_t* proof_len,
-                                  double* stats) {
+                                  double* stats, wf_aux_shard_builder_fn aux_builder = nullptr,
+                                  wf_aux_assertions_fn aux_assertions = nullptr, void* aux_user = nullptr) {
     std::vector<u8> out;
     int r;
     switch (o.ext) {
-        case 1: r = prove_sharded<1>(ctx, comm, air, local_cols, d_local, mont, log_n, o, out, stats); break;
-        case 2: r = prove_sharded<2>(ctx, comm, air, local_cols, d_local, mont, log_n, o, out, stats); break;
-        default: r = prove_sharded<3>(ctx, comm, air, local_cols, d_local, mont, log_n, o, out, stats); break;
+        case 1: r = prove_sharded<1>(ctx, comm, air, local_cols, d_local, mont, log_n, o, out, stats, aux_builder, aux_assertions, aux_user); break;
+        case 2: r = prove_sharded<2>(ctx, comm, air, local_cols, d_local, mont, log_n, o, out, stats, aux_builder, aux_assertions, aux_user); break;
+        default: r = prove_sharded<3>(ctx, comm, air, local_cols, d_local, mont, log_n, o, out, stats, aux_builder, aux_assertions, aux_user); break;
     }
     if (r != WF_OK) return r;
     if (out.size() > *proof_len) return wf_fail(ctx, WF_ERR_INVALID, "proof buffer too small (%zu needed)", out.size());
@@ -2324,10 +2449,12 @@ extern "C" int wf_host_shard_columns(uint32_t width, int world, int rank, uint32
 }
 // A sharded proof must not start unless every rank can go through with it: a rank that refused would otherwise leave the
 // others waiting in a collective. So each rank checks its own arguments (no device work), hashes what must be equal on
-// every rank, and one all-gather of (status, hash) decides for all of them.
-extern "C" int wf_prove_air_sharded(wf_ctx* ctx, const wf_comm* comm, const uint64_t* air_desc, size_t air_desc_len,
-                                    const uint64_t* const* local_cols, const uint64_t* d_local, int mont, uint32_t log_n,
-                                    const uint32_t* opts, uint8_t* proof, size_t* proof_len, double* stats) {
+// every rank, and one all-gather of (status, hash) decides for all of them. aux_entry: wf_prove_air_aux_sharded (the
+// description must have an aux segment), else wf_prove_air_sharded (it must not).
+static int prove_air_sharded_entry(wf_ctx* ctx, const wf_comm* comm, const uint64_t* air_desc, size_t air_desc_len,
+                                   const uint64_t* const* local_cols, const uint64_t* d_local, int mont, uint32_t log_n,
+                                   const uint32_t* opts, uint8_t* proof, size_t* proof_len, double* stats, bool aux_entry,
+                                   wf_aux_shard_builder_fn aux_builder, wf_aux_assertions_fn aux_assertions, void* aux_user) {
     if (!ctx || !comm || !comm->exchange || !comm->all_gather_host || !comm->all_reduce_sum || comm->world < 1 || comm->rank < 0 ||
         comm->rank >= comm->world)
         return wf_fail(ctx, WF_ERR_INVALID, "bad arguments");   // no communicator to agree over
@@ -2338,11 +2465,15 @@ extern "C" int wf_prove_air_sharded(wf_ctx* ctx, const wf_comm* comm, const uint
         if (!air_desc || !opts || !proof || !proof_len || log_n < 3 || log_n > 32) return wf_fail(ctx, WF_ERR_INVALID, "bad arguments");
         CKI(parse_options(ctx, opts, o));
         if (!parse_air_host(air_desc, air_desc_len, air)) return wf_fail(ctx, WF_ERR_INVALID, "malformed AIR description");
-        if (air.aw) return wf_fail(ctx, WF_ERR_UNSUPPORTED, "sharded proofs cover single-segment AIRs (this description has an auxiliary segment)");
+        if (!aux_entry && air.aw) return wf_fail(ctx, WF_ERR_UNSUPPORTED, "sharded proofs cover single-segment AIRs (this description has an auxiliary segment)");
+        if (aux_entry && !air.aw) return wf_fail(ctx, WF_ERR_INVALID, "the description has no auxiliary segment: use wf_prove_air_sharded");
+        if (aux_entry && !aux_builder) return wf_fail(ctx, WF_ERR_INVALID, "multi-segment AIR needs an aux trace builder");
+        if (air.aw * o.ext > 255) return wf_fail(ctx, WF_ERR_UNSUPPORTED, "at most 255 aux base columns (aux width x field extension)");
         CKI(sharded_shape_check(ctx, air, log_n, o, G, r));
         const size_t n = (size_t)1 << log_n;
         for (auto& col : air.periodic) if (col.size() > n) return wf_fail(ctx, WF_ERR_INVALID, "periodic column longer than the trace");
         CKI(validate_degrees(ctx, air.all_degrees(), n));
+        CKI(validate_assertions(ctx, air.aux_asserts, n, 3, "aux assertion"));
         CKI(validate_assertions(ctx, air.asserts, n, 1, "assertion"));
         u32 first = 0, count = 0;
         shard_columns(air.w, G, r, &first, &count);
@@ -2351,14 +2482,14 @@ extern "C" int wf_prove_air_sharded(wf_ctx* ctx, const wf_comm* comm, const uint
         return WF_OK;
     };
     const int mine = own_checks();
-    u64 hsh = 0xcbf29ce484222325ULL;   // FNV-1a over the description, log_n, the options and the world size
-    auto mix = [&](u64 v) { for (int i = 0; i < 8; i++) { hsh ^= (v >> (8 * i)) & 0xff; hsh *= 0x100000001b3ULL; } };
-    mix(air_desc ? air_desc_len : ~(u64)0);
-    for (size_t i = 0; air_desc && i < air_desc_len; i++) mix(air_desc[i]);
-    mix(log_n);
-    for (int i = 0; i < 9; i++) mix(opts ? opts[i] : ~(u64)0);
-    mix((u64)G);
-    struct Vote { int32_t status, pad; u64 hash; } v{mine, 0, hsh};
+    Fnv hsh;   // over the description, log_n, the options and the world size (and whether aux assertions are dynamic)
+    hsh.mix(air_desc ? air_desc_len : ~(u64)0);
+    for (size_t i = 0; air_desc && i < air_desc_len; i++) hsh.mix(air_desc[i]);
+    hsh.mix(log_n);
+    for (int i = 0; i < 9; i++) hsh.mix(opts ? opts[i] : ~(u64)0);
+    hsh.mix((u64)G);
+    if (aux_entry) hsh.mix(aux_assertions ? 1 : 0);
+    struct Vote { int32_t status, pad; u64 hash; } v{mine, 0, hsh.h};
     std::vector<Vote> all(G);
     if (comm->all_gather_host(comm->user, &v, all.data(), sizeof(Vote)) != 0) return wf_fail(ctx, WF_ERR_STATE, "all_gather_host callback failed");
     for (int q = 0; q < G; q++) {   // the lowest refusing rank's status, on every rank
@@ -2368,8 +2499,24 @@ extern "C" int wf_prove_air_sharded(wf_ctx* ctx, const wf_comm* comm, const uint
         return wf_fail(ctx, all[q].status, "rank %d refused the sharded proof%s", q, own.c_str());
     }
     for (int q = 0; q < G; q++)
-        if (all[q].hash != hsh) return wf_fail(ctx, WF_ERR_INVALID, "ranks %d and %d were given different AIR descriptions, trace lengths, options or world sizes", r, q);
-    return prove_sharded_dispatch(ctx, comm, air, local_cols, d_local, mont, log_n, o, proof, proof_len, stats);
+        if (all[q].hash != hsh.h)
+            return wf_fail(ctx, WF_ERR_INVALID, "ranks %d and %d were given different AIR descriptions, trace lengths, options or world sizes%s", r, q,
+                           aux_entry ? " (or only one of them an aux assertion callback)" : "");
+    return prove_sharded_dispatch(ctx, comm, air, local_cols, d_local, mont, log_n, o, proof, proof_len, stats, aux_builder, aux_assertions,
+                                  aux_user);
+}
+extern "C" int wf_prove_air_sharded(wf_ctx* ctx, const wf_comm* comm, const uint64_t* air_desc, size_t air_desc_len,
+                                    const uint64_t* const* local_cols, const uint64_t* d_local, int mont, uint32_t log_n,
+                                    const uint32_t* opts, uint8_t* proof, size_t* proof_len, double* stats) {
+    return prove_air_sharded_entry(ctx, comm, air_desc, air_desc_len, local_cols, d_local, mont, log_n, opts, proof, proof_len, stats, false,
+                                   nullptr, nullptr, nullptr);
+}
+extern "C" int wf_prove_air_aux_sharded(wf_ctx* ctx, const wf_comm* comm, const uint64_t* air_desc, size_t air_desc_len,
+                                        const uint64_t* const* local_cols, const uint64_t* d_local, int mont, uint32_t log_n,
+                                        const uint32_t* opts, wf_aux_shard_builder_fn aux_builder, wf_aux_assertions_fn aux_assertions,
+                                        void* aux_user, uint8_t* proof, size_t* proof_len, double* stats) {
+    return prove_air_sharded_entry(ctx, comm, air_desc, air_desc_len, local_cols, d_local, mont, log_n, opts, proof, proof_len, stats, true,
+                                   aux_builder, aux_assertions, aux_user);
 }
 extern "C" int wf_prove_fib(wf_ctx* ctx, const uint64_t* const* trace_cols, int mont, uint32_t k, uint32_t log_n,
                             const uint64_t* results, const uint32_t* opts, uint8_t* proof, size_t* proof_len) {

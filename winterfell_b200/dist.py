@@ -130,7 +130,7 @@ def sharded_trace_commit(backend, hash_id, local_cols, ncols_total, log_n, log_b
 
 # --------------------------------------------------------------------------------------------------
 # One proof sharded over the ranks of a torch.distributed group (wf_prove_fib_sharded, wf_prove_air_sharded,
-# include/winterfell_b200.h).
+# wf_prove_air_aux_sharded, include/winterfell_b200.h).
 # The library does all arithmetic and orchestration; this module only supplies the three collectives of `wf_comm`.
 # --------------------------------------------------------------------------------------------------
 import ctypes as C
@@ -286,23 +286,14 @@ def prove_fib_sharded(ctx, comm, local_trace, k, log_n, results, opts, out_buf=N
     if comm.error is not None:
         raise comm.error
     if stats is not None:
-        stats.update({"bytes_sent": st[0], "exchange_ms": st[1], "collectives": st[2], "small_collective_ms": st[3], "sharded_fri_layers": st[4],
-                      "bytes_overlapped": st[5], "peer_push": st[6]})
+        stats.update(_sharded_stats(st))
     return buf[: ln.value].tobytes()
 
 
-def prove_air_sharded(ctx, comm, desc, local_trace, log_n, opts, mont=False, device_ptr=None, stats=None, out_buf=None):
-    """One proof of a single-segment AIR description (as Context.prove_air) over comm.world GPUs. local_trace: this rank's
-    columns (wf.shard_columns(width, world, rank)) as a [count, n] uint64 host array, or device_ptr = raw pointer to the same
-    block column-major in HBM; a rank that owns no column passes an empty array or None. desc, log_n and opts are the whole
-    proof's. Returns the proof bytes (identical on every rank). Every rank raises when any rank refuses the arguments."""
-    L = wf.lib()
-    d_ = np.ascontiguousarray(desc, dtype=np.uint64)
-    o_ = np.ascontiguousarray(opts, dtype=np.uint32)
-    buf = out_buf if out_buf is not None else np.zeros(1 << 23, dtype=np.uint8)
-    ln = C.c_size_t(buf.size)
-    st = (C.c_double * 8)()
-    ptrs, dptr, wrong = None, None, None
+def _local_columns(comm, d_, local_trace, log_n, device_ptr):
+    """This rank's main columns for wf_prove_air[_aux]_sharded: (column pointers, device pointer, what is wrong with the block
+    or None, the array the pointers point into)."""
+    ptrs, dptr, wrong, a = None, None, None, None
     if device_ptr is not None:
         dptr = C.c_void_p(device_ptr)
     elif local_trace is not None and len(local_trace):
@@ -318,6 +309,26 @@ def prove_air_sharded(ctx, comm, desc, local_trace, log_n, opts, mont=False, dev
             # agreement step and every rank returns the error instead of waiting on this one
             wrong = f"rank {comm.rank} passed a [{a.shape[0]}, {a.shape[1]}] block, owns {count} columns of {1 << log_n} rows"
             ptrs = None if count else ptrs
+    return ptrs, dptr, wrong, a
+
+
+def _sharded_stats(st):
+    return {"bytes_sent": st[0], "exchange_ms": st[1], "collectives": st[2], "small_collective_ms": st[3], "sharded_fri_layers": st[4],
+            "bytes_overlapped": st[5], "peer_push": st[6]}
+
+
+def prove_air_sharded(ctx, comm, desc, local_trace, log_n, opts, mont=False, device_ptr=None, stats=None, out_buf=None):
+    """One proof of a single-segment AIR description (as Context.prove_air) over comm.world GPUs. local_trace: this rank's
+    columns (wf.shard_columns(width, world, rank)) as a [count, n] uint64 host array, or device_ptr = raw pointer to the same
+    block column-major in HBM; a rank that owns no column passes an empty array or None. desc, log_n and opts are the whole
+    proof's. Returns the proof bytes (identical on every rank). Every rank raises when any rank refuses the arguments."""
+    L = wf.lib()
+    d_ = np.ascontiguousarray(desc, dtype=np.uint64)
+    o_ = np.ascontiguousarray(opts, dtype=np.uint32)
+    buf = out_buf if out_buf is not None else np.zeros(1 << 23, dtype=np.uint8)
+    ln = C.c_size_t(buf.size)
+    st = (C.c_double * 8)()
+    ptrs, dptr, wrong, _keep = _local_columns(comm, d_, local_trace, log_n, device_ptr)
     r = L.wf_prove_air_sharded(ctx.h, C.byref(comm.struct), d_.ctypes.data_as(wf.u64p), d_.size, ptrs, dptr, int(mont), log_n,
                                o_.ctypes.data_as(C.POINTER(C.c_uint32)), buf.ctypes.data_as(wf.u8p), C.byref(ln), st)
     if comm.error is not None:
@@ -326,8 +337,65 @@ def prove_air_sharded(ctx, comm, desc, local_trace, log_n, opts, mont=False, dev
         raise wf.WfError(f"error {r}: {wrong}")
     ctx.check(r)
     if stats is not None:
-        stats.update({"bytes_sent": st[0], "exchange_ms": st[1], "collectives": st[2], "small_collective_ms": st[3], "sharded_fri_layers": st[4],
-                      "bytes_overlapped": st[5], "peer_push": st[6]})
+        stats.update(_sharded_stats(st))
+    return buf[: ln.value].tobytes()
+
+
+def prove_air_aux_sharded(ctx, comm, desc, local_trace, log_n, opts, builder, values_fn=None, mont=False, device_ptr=None, stats=None,
+                          out_buf=None):
+    """One proof of a two-segment AIR description (as Context.prove_air_aux, or prove_air_aux_dyn with values_fn) over
+    comm.world GPUs. The main columns are passed as in prove_air_sharded. builder(rand [nr, d], first_col, num_cols) ->
+    [num_cols, n, d]: the aux E columns [first_col, first_col + num_cols) this rank owns components of (wf_prove_air_aux_sharded;
+    not called on a rank that owns no aux column; must be deterministic: an E column split between two ranks is built by
+    both). values_fn(rand, values [nv, d]) -> values: the aux assertion values (Air::get_aux_assertions), called on every
+    rank, which must all return the same. An exception inside a callback makes every rank fail: the rank it happened on
+    re-raises it, the others raise WfError. Returns the proof bytes (identical on every rank); stats also gets "callback_ms",
+    the time this rank spent in the two callbacks."""
+    L = wf.lib()
+    d_ = np.ascontiguousarray(desc, dtype=np.uint64)
+    o_ = np.ascontiguousarray(opts, dtype=np.uint32)
+    buf = out_buf if out_buf is not None else np.zeros(1 << 23, dtype=np.uint8)
+    ln = C.c_size_t(buf.size)
+    st = (C.c_double * 8)()
+    ptrs, dptr, wrong, _keep = _local_columns(comm, d_, local_trace, log_n, device_ptr)
+    _, nr, nv = wf.aux_shape(d_)
+    d, n = int(o_[3]) if o_.size > 3 else 1, 1 << log_n
+    raised = []
+
+    def guard(fn):
+        def wrapped(*args):
+            try:
+                fn(*args)
+                return 0
+            except Exception as e:  # must not unwind through the C caller; the library's agreement step fails every rank
+                raised.append(e)
+                return 1
+        return wrapped
+
+    def cb_build(_user, rand_p, first_col, num_cols, out_p):
+        rand = np.ctypeslib.as_array(rand_p, shape=(nr, d)).copy() if nr else np.zeros((0, d), dtype=np.uint64)
+        aux = np.ascontiguousarray(builder(rand, first_col, num_cols), dtype=np.uint64).reshape(num_cols, n, d)
+        np.ctypeslib.as_array(out_p, shape=(num_cols, n, d))[:] = aux
+
+    def cb_values(_user, rand_p, val_p):
+        rand = np.ctypeslib.as_array(rand_p, shape=(nr, d)).copy() if nr else np.zeros((0, d), dtype=np.uint64)
+        vals = np.ctypeslib.as_array(val_p, shape=(nv, d))
+        vals[:] = np.ascontiguousarray(values_fn(rand, vals.copy()), dtype=np.uint64).reshape(nv, d)
+
+    fb = wf.AUX_SHARD_BUILDER(guard(cb_build)) if builder is not None else wf.AUX_SHARD_BUILDER()   # (NULL: refused)
+    fv = wf.AUX_BUILDER(guard(cb_values)) if values_fn is not None else wf.AUX_BUILDER()
+    r = L.wf_prove_air_aux_sharded(ctx.h, C.byref(comm.struct), d_.ctypes.data_as(wf.u64p), d_.size, ptrs, dptr, int(mont), log_n,
+                                   o_.ctypes.data_as(C.POINTER(C.c_uint32)), fb, fv, None, buf.ctypes.data_as(wf.u8p), C.byref(ln), st)
+    if comm.error is not None:
+        raise comm.error
+    if raised:
+        raise raised[0]
+    if r != wf.WF_OK and wrong:
+        raise wf.WfError(f"error {r}: {wrong}")
+    ctx.check(r)
+    if stats is not None:
+        stats.update(_sharded_stats(st))
+        stats["callback_ms"] = st[7]
     return buf[: ln.value].tobytes()
 
 
